@@ -4,6 +4,7 @@
 
   python bench.py [--gpus N --steps K --warmup W]            this repo's CUDA path
   python bench.py --impl reference [...]                     the reference's CPU path (oracle port)
+  python bench.py [...] --dump-outputs DIR                   also write the last timed step's output to DIR/*.npy
   torchrun-style launch for N > 1 (one rank per GPU, RANK/LOCAL_RANK/WORLD_SIZE from env).
 
 One "step" = one synthetic mono file of `--chunks-per-step` 2-second chunks per GPU pushed through
@@ -24,6 +25,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (no __pycache__ of its imports)
 
 SR = 22050
 CHUNK, OVERLAP = 44100, 2052
@@ -228,6 +230,31 @@ def step_samples(args):
     return (args.chunks_per_step - 1) * HOP + CHUNK
 
 
+DUMP_MAX_BYTES = 64 << 20
+DUMP_WINDOW = 4096                  # consecutive output samples per sampled window
+DUMP_WINDOWS = 1024                 # windows per channel: 2 x 1024 x 4096 float32 = 32 MB
+
+
+def dump_outputs(y, out_dir):
+    """Write the restored stereo `[2, M]` of the last timed step under `out_dir`, so that two builds run with the same
+    arguments (hence the same inputs) can be compared output for output.  Up to 64 MB it is written whole as
+    `restored.npy`; a larger output as `restored_windows.npy` `[2, 1024, 4096]`: windows at the first and last sample and at
+    1022 starts drawn from a fixed seed (the same positions for the same M), with the starts, as sample indices, in
+    `restored_window_starts.npy` (float64)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    if y.numel() * 4 <= DUMP_MAX_BYTES:
+        np.save(os.path.join(out_dir, "restored.npy"), y.float().cpu().numpy())
+        return
+    m = y.shape[1]
+    g = torch.Generator().manual_seed(0)
+    drawn = torch.randint(0, m - DUMP_WINDOW + 1, (DUMP_WINDOWS - 2,), generator=g)
+    starts = torch.cat([torch.tensor([0, m - DUMP_WINDOW]), drawn]).sort().values
+    idx = (starts[:, None] + torch.arange(DUMP_WINDOW)).to(y.device)
+    np.save(os.path.join(out_dir, "restored_windows.npy"), y[:, idx].float().cpu().numpy())
+    np.save(os.path.join(out_dir, "restored_window_starts.npy"), starts.double().numpy())
+
+
 def flush_l2(buf):
     buf.add_(1.0)     # read + write 512 MB: everything older leaves the 126 MB L2
 
@@ -402,8 +429,7 @@ def run_b200(args, rank, world, local_rank):
                             return_device=True, streams=args.streams)
 
     for _ in range(args.warmup):
-        y = step_resident()
-    assert y.shape == (2, 2 * n)
+        step_resident()
     sync_all()
 
     # ---- timed region: K steps, inputs resident in HBM, CUDA events on the launching stream
@@ -425,6 +451,9 @@ def run_b200(args, rank, world, local_rank):
     _lib.check(L.ar_profile_read(p_ms, p_fl, p_ln, ncat))
     L.ar_profile_enable(0)
     clocks = sampler.finish()
+    assert y.shape == (2, 2 * n)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(y, args.dump_outputs)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     t_s = float(ms.item()) / 1e3
@@ -549,7 +578,13 @@ def main():
     ap.add_argument("--cpu-chunks", type=int, default=32, help="chunks in the bounded CPU sample (32 = 61 s of audio, about 11 s on 16 host cores)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the per-config lines (BASELINE configs 1-4) and the torch-eager same-GPU bar")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the restored stereo of the last one "
+                    "(rank 0; whole up to 64 MB, else a fixed seeded sample of windows) to DIR as float32 .npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the output of the CUDA path (--impl b200)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

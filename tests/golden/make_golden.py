@@ -1,7 +1,7 @@
 """Generate tests/golden/*.npz by running the UNMODIFIED reference on CPU.
 
-Run in the build container only (needs /root/reference, which does not exist on the GPU
-box):   python tests/golden/make_golden.py
+Needs a checkout of the original project (its `src/` package):
+        python tests/golden/make_golden.py <original-project-dir>
 
 What it pins
   * the oracle `state_dict` factory has exactly the reference key set / shapes
@@ -24,8 +24,9 @@ sys.dont_write_bytecode = True
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-REF = "/root/reference"
-sys.path.insert(0, REF)
+if len(sys.argv) != 2:
+    sys.exit("usage: python tests/golden/make_golden.py <original-project-dir>")
+sys.path.insert(0, os.path.abspath(sys.argv[1]))
 sys.modules.setdefault("soundfile", types.ModuleType("soundfile"))  # audio_processing.py:3
 
 from src.models.denoiser import AudioDenoiser                      # noqa: E402  (reference)

@@ -1,7 +1,7 @@
 """Golden vectors for the degradation generator, produced by the UNMODIFIED reference function
-(`simulate_vinyl_artifacts`, /root/reference/src/utils/audio_processing.py:122-226) in the build container:
+(`simulate_vinyl_artifacts`, src/utils/audio_processing.py:122-226 of the original project):
 
-    python tests/golden/make_golden_degrade.py      ->  tests/golden/golden_degrade_v1.npz
+    python tests/golden/make_golden_degrade.py <original-project-dir>      ->  tests/golden/golden_degrade_v1.npz
 
 `soundfile` (imported at audio_processing.py:3, not installed here) is stubbed; nothing else is touched.  Inputs are
 regenerated from the seeds stored in the file; both global generators the reference uses are seeded per case
@@ -29,8 +29,10 @@ def make_input(seed, C, N):
 
 
 def main():
+    if len(sys.argv) != 2:
+        sys.exit("usage: python tests/golden/make_golden_degrade.py <original-project-dir>")
     sys.modules.setdefault("soundfile", types.ModuleType("soundfile"))
-    sys.path.insert(0, "/root/reference")
+    sys.path.insert(0, os.path.abspath(sys.argv[1]))
     from src.utils.audio_processing import simulate_vinyl_artifacts
     import scipy
     out = {"scipy_version": np.array(scipy.__version__), "n_cases": np.array(len(CASES))}

@@ -235,3 +235,32 @@ def test_restore_stream_matches_per_file_restore(pipe):
     assert list(pipe.restore_stream(iter([]))) == []
     with pytest.raises(ValueError):
         list(pipe.restore_stream(iter(files), return_device=True))
+
+
+def test_bench_dump_outputs_is_the_timed_restore(tmp_path):
+    """`bench.py --dump-outputs` at a small geometry, no warm-up: the JSON line reports the requested number of timed steps,
+    and the dumped array is what `restore(mode="chunked")` returns for the bench's seeded input and weights."""
+    import json
+    import os
+    import subprocess
+    import sys
+    from oracle.weights import make_state_dict
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    sys.path.insert(0, root)
+    import bench
+    chunks = 4
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "2", "--warmup", "0", "--chunks-per-step",
+                          str(chunks), "--batch-chunks", str(chunks), "--no-cpu-baseline", "--no-secondary",
+                          "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=900)
+    assert out.returncode == 0, out.stdout[-2000:] + out.stderr[-2000:]
+    line = json.loads(out.stdout.strip().splitlines()[-1])
+    assert line["steps"] == 2 and line["warmup"] == 0 and line["parity"]["pass"]
+    assert sorted(os.listdir(tmp_path)) == ["restored.npy"]
+    dumped = np.load(tmp_path / "restored.npy")
+    sds = {n: make_state_dict(n) for n in oracle.MODEL_NAMES}
+    p = RestorationPipeline.from_state_dicts(sds["denoiser"], sds["super_resolution"], sds["stereo"], "cuda")
+    n = (chunks - 1) * bench.HOP + bench.CHUNK
+    want = p.restore(bench.synth_audio(n, 1000, "cuda:0"), mode="chunked", chunk_size=bench.CHUNK, overlap=bench.OVERLAP,
+                     batch_chunks=chunks)
+    assert dumped.dtype == np.float32 and dumped.shape == (2, 2 * n)
+    assert np.array_equal(dumped, want.cpu().numpy())

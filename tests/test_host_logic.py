@@ -224,6 +224,40 @@ def test_bench_algorithmic_constants():
     assert bench.CONV_GFLOP_PER_AUDIO_S - bench.CONV_GFLOP_PER_AUDIO_S_FUSED_SCAN == pytest.approx(2e-9 * 32768 * 44100, rel=1e-6)
 
 
+def test_bench_dump_outputs_whole_or_fixed_sample(tmp_path):
+    """`--dump-outputs`: an output up to 64 MB is written whole; a larger one as windows at fixed seeded positions (the first
+    and last sample included) that hold exactly the output's samples, the same positions on every call, under 64 MB."""
+    sys.path.insert(0, ROOT)
+    import bench
+    small = torch.randn(2, 1000)
+    bench.dump_outputs(small, str(tmp_path / "small"))
+    assert sorted(os.listdir(tmp_path / "small")) == ["restored.npy"]
+    assert np.array_equal(np.load(tmp_path / "small" / "restored.npy"), small.numpy())
+    m = bench.DUMP_MAX_BYTES // 8 + 1000                        # [2, m] float32 just over 64 MB
+    big = torch.randn(2, m, generator=torch.Generator().manual_seed(5))
+    for d in ("a", "b"):
+        bench.dump_outputs(big, str(tmp_path / d))
+    names = ["restored_window_starts.npy", "restored_windows.npy"]
+    assert sorted(os.listdir(tmp_path / "a")) == names
+    w, starts = np.load(tmp_path / "a" / names[1]), np.load(tmp_path / "a" / names[0])
+    assert w.dtype == np.float32 and starts.dtype == np.float64
+    assert w.shape == (2, bench.DUMP_WINDOWS, bench.DUMP_WINDOW) and w.nbytes + starts.nbytes <= bench.DUMP_MAX_BYTES
+    assert starts[0] == 0 and starts[-1] == m - bench.DUMP_WINDOW and np.all(np.diff(starts) >= 0)
+    for i in (0, 1, len(starts) // 2, len(starts) - 1):
+        s = int(starts[i])
+        assert np.array_equal(w[:, i], big[:, s:s + bench.DUMP_WINDOW].numpy())
+    for name in names:
+        assert np.array_equal(np.load(tmp_path / "a" / name), np.load(tmp_path / "b" / name))
+
+
+@pytest.mark.parametrize("argv", [["--steps", "0"], ["--warmup", "-1"], ["--impl", "reference", "--dump-outputs", "out"]])
+def test_bench_rejects_bad_arguments(argv, tmp_path):
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *argv], capture_output=True, text=True, cwd=tmp_path,
+                         timeout=300)
+    assert out.returncode == 2 and "error" in out.stderr, out.stderr[-2000:]
+    assert not (tmp_path / "out").exists()
+
+
 def test_butter_design_matches_scipy():
     """`ar_butter` (host function of the C-ABI) against scipy.signal.butter at the three designs the reference uses
     (audio_processing.py:196, 208, 220) and a few others."""
