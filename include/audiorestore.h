@@ -166,6 +166,24 @@ int ar_pcm16_to_float(const int16_t* pcm, int channels, int64_t n, float* y, voi
 #define AR_PCM_F64 6
 int ar_pcm_to_float(const void* raw, int format, int channels, int64_t n, float* y, void* stream);
 
+/* FLAC input for the same front end: sf.read of a .flac file (audio_processing.py:24), decoded on the device (RFC 9639).
+ *   ar_flac_workspace_bytes : device scratch ar_flac_decode needs for `nbytes` bytes of frame data
+ *   ar_flac_decode          : frames[nbytes] = the frame section of one stream (DEVICE bytes after the metadata blocks);
+ *                             channels / bps / sample_rate / min_block / max_block / total_samples are the STREAMINFO
+ *                             fields (total_samples 0 = unknown) -> planar fp32 y[channels][n] (row stride n),
+ *                             x / 2^(bps-1) as soundfile's float32 read scales it (bit-exact for bps <= 24; 32-bit through
+ *                             __int2float_rn, as AR_PCM_S32).  *n_out receives the samples per channel; y == NULL only
+ *                             counts them (for total_samples 0).  Frames are found by a frame-parallel index of sync codes,
+ *                             chained from byte 0 and decoded one thread per frame.  Synchronises `stream` to read the
+ *                             frame table back (a loader that runs once per file).  A malformed stream -- CRC-8 / CRC-16
+ *                             mismatch, reserved code, truncation, a change of rate / depth / channels mid-stream, frames
+ *                             that disagree with total_samples -- returns AR_ERR_INVALID with a message naming the frame
+ *                             index and byte offset in `frames`.  MD5 is not checked (libFLAC's default too). */
+int ar_flac_workspace_bytes(int64_t nbytes, size_t* bytes);
+int ar_flac_decode(const uint8_t* frames, int64_t nbytes, int channels, int bps, int sample_rate, int min_block, int max_block,
+                   int64_t total_samples, float* y, int64_t n, int64_t* n_out, void* workspace, size_t workspace_bytes,
+                   void* stream);
+
 /* Synthetic 78 rpm degradation generator (simulate_vinyl_artifacts, audio_processing.py:122-226; SURVEY.md 8f n4).
  * The random draws (np.random levels / pop plan, torch.randn noise tensors) stay with the caller; these entry points
  * are the deterministic arithmetic, rows = channels (or any batch of equal-length rows), all device fp32 [rows][n]:

@@ -1,7 +1,7 @@
 """Audio helpers on the restoration path (reference: src/utils/audio_processing.py).
 
 What inference needs -- `normalize_audio` (device kernel, no host syncs), `chunk_audio` (the reference's chunk
-vocabulary), small WAV load/save helpers so `restore_audio` works without `soundfile` (not installed in this image) --
+vocabulary), small WAV load/save helpers and a GPU FLAC decoder so `restore_audio` works without `soundfile` --
 plus the synthetic degradation generator `simulate_vinyl_artifacts` (SURVEY.md 8f n4) that produces the path's
 78 rpm-like inputs, with its pops and zero-phase Butterworth filters on the GPU.
 """
@@ -205,14 +205,18 @@ def simulate_vinyl_artifacts(audio: torch.Tensor, sample_rate: int, impulse_rate
 # ----------------------------------------------------------------------------- minimal WAV I/O
 def _read_wav(path: str):
     """Host read of an audio file as `[C, N]` float32 (the reference's `sf.read(..., dtype='float32')`,
-    audio_processing.py:24): soundfile when it is installed, else the RIFF/WAVE reader of this module (8 / 16 / 24 / 32-bit
-    integer PCM, 32 / 64-bit IEEE float, plain or WAVE_FORMAT_EXTENSIBLE)."""
+    audio_processing.py:24): soundfile when it is installed, else FLAC through the device decoder (`decode_flac_cuda`,
+    returned on the host) and WAV through the RIFF/WAVE reader of this module (8 / 16 / 24 / 32-bit integer PCM,
+    32 / 64-bit IEEE float, plain or WAVE_FORMAT_EXTENSIBLE)."""
     try:
         import soundfile as sf  # optional
         data, sr = sf.read(path, always_2d=True, dtype="float32")
         return torch.from_numpy(np.ascontiguousarray(data.T)), sr
     except ImportError:
         pass
+    if is_flac(path):                                             # decoded on the GPU (ar_flac_decode)
+        info = flac_info(path)
+        return decode_flac_cuda(_upload_frames(path, info, "cuda"), info).cpu(), info["sample_rate"]
     fmt, nch, sr, frames, offset = wav_info(path)
     width = _PCM_WIDTH[fmt]
     with open(path, "rb") as f:
@@ -316,13 +320,133 @@ def decode_pcm_cuda(raw: torch.Tensor, fmt: int, channels: int, frames: int) -> 
     return planar
 
 
+# ----------------------------------------------------------------------------- FLAC
+_FLAC_SKIPPED_BLOCKS = (1, 2, 3, 4, 5, 6)     # PADDING, APPLICATION, SEEKTABLE, VORBIS_COMMENT, CUESHEET, PICTURE
+
+
+def _flac_start(head: bytes) -> int:
+    """Offset of the `fLaC` marker: 0, or past a leading ID3v2 tag (10-byte header, syncsafe size, optional footer)."""
+    if head[:3] == b"ID3" and len(head) >= 10:
+        size = (head[6] << 21) | (head[7] << 14) | (head[8] << 7) | head[9]
+        return 10 + size + (10 if head[5] & 0x10 else 0)
+    return 0
+
+
+def is_flac(path: str) -> bool:
+    """True when the file's content is a FLAC stream (optionally behind an ID3v2 tag), whatever its extension."""
+    with open(path, "rb") as f:
+        head = f.read(10)
+        f.seek(_flac_start(head))
+        return f.read(4) == b"fLaC"
+
+
+def flac_info(path: str) -> dict:
+    """Host parse of a FLAC container (RFC 9639): an optional leading ID3v2 tag, the `fLaC` marker, then the metadata
+    blocks -- STREAMINFO required, PADDING / APPLICATION / SEEKTABLE / VORBIS_COMMENT / CUESHEET / PICTURE skipped.
+    Returns {channels, bps, sample_rate, total_samples (0 = unknown), min_block, max_block, offset (byte offset of the
+    first frame), nbytes (bytes of frame data)}; raises RuntimeError for anything that is not a well-formed FLAC header."""
+    import os
+    size = os.path.getsize(path)
+    with open(path, "rb") as f:
+        pos = _flac_start(f.read(10))
+        f.seek(pos)
+        if f.read(4) != b"fLaC":
+            raise RuntimeError(f"{path}: not a FLAC file")
+        pos += 4
+        info = None
+        while True:
+            hdr = f.read(4)
+            if len(hdr) < 4:
+                raise RuntimeError(f"{path}: truncated FLAC metadata block header")
+            last, btype, length = hdr[0] >> 7, hdr[0] & 0x7F, int.from_bytes(hdr[1:4], "big")
+            pos += 4
+            if pos + length > size:
+                raise RuntimeError(f"{path}: truncated FLAC metadata block (type {btype})")
+            if btype == 0:
+                if length != 34 or info is not None:
+                    raise RuntimeError(f"{path}: malformed STREAMINFO block")
+                b = f.read(34)
+                v = int.from_bytes(b[10:18], "big")
+                info = {"min_block": int.from_bytes(b[0:2], "big"), "max_block": int.from_bytes(b[2:4], "big"),
+                        "sample_rate": v >> 44, "channels": ((v >> 41) & 7) + 1, "bps": ((v >> 36) & 31) + 1,
+                        "total_samples": v & ((1 << 36) - 1)}
+            elif btype in _FLAC_SKIPPED_BLOCKS or 7 <= btype < 127:
+                f.seek(length, 1)
+            else:
+                raise RuntimeError(f"{path}: invalid FLAC metadata block type {btype}")
+            pos += length
+            if btype != 0 and info is None:
+                raise RuntimeError(f"{path}: FLAC metadata does not start with STREAMINFO")
+            if last:
+                break
+    if info["sample_rate"] == 0 or info["bps"] < 4 or info["min_block"] < 1 or info["max_block"] < info["min_block"]:
+        raise RuntimeError(f"{path}: STREAMINFO holds a reserved value (rate {info['sample_rate']}, {info['bps']} bits, "
+                           f"block sizes {info['min_block']}..{info['max_block']})")
+    info["offset"] = pos
+    info["nbytes"] = size - pos
+    return info
+
+
+def _upload_frames(path: str, info: dict, device) -> torch.Tensor:
+    """The frame bytes of a FLAC file, read into pinned memory and copied to `device` (uint8)."""
+    host = torch.empty(info["nbytes"], dtype=torch.uint8).pin_memory()
+    with open(path, "rb") as f:
+        f.seek(info["offset"])
+        got = f.readinto(host.numpy())
+    if got != host.numel():
+        raise RuntimeError(f"{path}: file changed while reading")
+    return host.to(torch.device(device), non_blocking=True)
+
+
+def decode_flac_cuda(raw: torch.Tensor, info: dict) -> torch.Tensor:
+    """The frame bytes of a FLAC stream (uint8 CUDA tensor, everything after the metadata blocks) and its `flac_info` ->
+    planar `[channels, N]` float32, x / 2^(bps-1) as soundfile's float32 read (`ar_flac_decode`; bit-exact for
+    bps <= 24).  Raises RuntimeError naming the frame and its byte offset in the file for a malformed stream."""
+    if not raw.is_cuda or raw.dtype != torch.uint8 or raw.dim() != 1:
+        raise RuntimeError("decode_flac_cuda: expected a 1-D uint8 CUDA tensor -- this build has no CPU fallback")
+    raw = raw.contiguous()
+    L = _lib.lib()
+    need = C.c_size_t()
+    _lib.check(L.ar_flac_workspace_bytes(raw.numel(), C.byref(need)))
+    n_out = C.c_int64()
+    with torch.cuda.device(raw.device):
+        stream = torch.cuda.current_stream(raw.device).cuda_stream
+        ws = torch.empty(need.value, dtype=torch.uint8, device=raw.device)
+        args = (raw.data_ptr(), raw.numel(), info["channels"], info["bps"], info["sample_rate"], info["min_block"],
+                info["max_block"], info["total_samples"])
+
+        def run(y, n):
+            try:
+                _lib.check(L.ar_flac_decode(*args, y.data_ptr() if y is not None else None, n, C.byref(n_out),
+                                            ws.data_ptr(), need.value, stream))
+            except RuntimeError as e:
+                off = info.get("offset")
+                raise RuntimeError(str(e) + (f" (frame data starts at byte {off} of the file)" if off else "")) from None
+
+        n = info["total_samples"]
+        if n == 0:                                                # unknown length: count the samples first
+            run(None, 0)
+            n = n_out.value
+        y = torch.empty((info["channels"], n), dtype=torch.float32, device=raw.device)
+        run(y, n)
+    return y
+
+
 def load_audio_cuda(file_path: str, sample_rate: int = 22050, device="cuda"):
     """`load_audio(..., mono=True)` with the arithmetic on the GPU (SURVEY.md 8f n1): the `data` chunk of a WAV file --
     8 / 16 / 24 / 32-bit integer PCM, 32 / 64-bit IEEE float, plain or WAVE_FORMAT_EXTENSIBLE -- is uploaded as the raw
     bytes it is (a 16-bit file costs half the H2D bytes of float32) from pinned memory, then decoded, mixed to mono and
-    resampled on the device.  Other containers go through `_read_wav` (soundfile, when installed) and only the mix and
-    the resampling run on the GPU.  Returns (audio [1,N] float32 CUDA, sample_rate)."""
+    resampled on the device.  A FLAC file (recognised by its content, not its extension) uploads its compressed frame
+    bytes the same way and is decoded on the device (`decode_flac_cuda`).  Other containers go through `_read_wav`
+    (soundfile, when installed) and only the mix and the resampling run on the GPU.  Returns (audio [1,N] float32 CUDA,
+    sample_rate)."""
     dev = torch.device(device)
+    if is_flac(file_path):
+        info = flac_info(file_path)
+        planar = decode_flac_cuda(_upload_frames(file_path, info, dev), info)
+        if planar.shape[1] < 1:
+            raise RuntimeError(f"{file_path}: no audio frames")
+        return resample_mono_cuda(planar, info["sample_rate"], sample_rate), sample_rate
     try:
         fmt, nch, sr, frames, offset = wav_info(file_path)
     except RuntimeError:

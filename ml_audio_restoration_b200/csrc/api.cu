@@ -19,6 +19,10 @@ int launch_resample_mono(const float* x, int channels, long long n, int orig_sr,
                          cudaStream_t stream);
 int launch_pcm16(const short* pcm, int channels, long long n, float* y, cudaStream_t stream);
 int launch_pcm_decode(const void* raw, int format, int channels, long long n, float* y, cudaStream_t stream);
+int flac_workspace_bytes(long long nbytes, size_t* bytes);
+int flac_decode(const unsigned char* data, long long nbytes, int channels, int bps, int sample_rate, int min_block,
+                int max_block, long long total_samples, float* y, long long n, long long* n_out, void* ws, size_t ws_bytes,
+                cudaStream_t stream);
 int butter(int order, double wn, int highpass, double* b, double* a);
 int launch_vinyl_mix(const float* audio, const float* noise, float level, const void* pops, int n_pops, int sample_rate,
                      float* y, int rows, long long n, cudaStream_t stream);
@@ -71,6 +75,16 @@ int ar_pcm16_to_float(const int16_t* pcm, int channels, int64_t n, float* y, voi
 }
 int ar_pcm_to_float(const void* raw, int format, int channels, int64_t n, float* y, void* stream) {
   return ar::launch_pcm_decode(raw, format, channels, n, y, reinterpret_cast<cudaStream_t>(stream));
+}
+int ar_flac_workspace_bytes(int64_t nbytes, size_t* bytes) { return ar::flac_workspace_bytes(nbytes, bytes); }
+int ar_flac_decode(const uint8_t* frames, int64_t nbytes, int channels, int bps, int sample_rate, int min_block, int max_block,
+                   int64_t total_samples, float* y, int64_t n, int64_t* n_out, void* workspace, size_t workspace_bytes,
+                   void* stream) {
+  long long got = 0;
+  const int rc = ar::flac_decode(frames, nbytes, channels, bps, sample_rate, min_block, max_block, total_samples, y, n, &got,
+                                 workspace, workspace_bytes, reinterpret_cast<cudaStream_t>(stream));
+  if (n_out) *n_out = got;
+  return rc;
 }
 int ar_butter(int order, double wn, int highpass, double* b, double* a) { return ar::butter(order, wn, highpass, b, a); }
 int ar_vinyl_mix(const float* audio, const float* surface_noise, float surface_level, const ar_pop_t* pops, int n_pops,

@@ -27,7 +27,7 @@ import math
 import torch
 
 from . import _lib
-from .audio_processing import load_audio, load_audio_cuda, save_audio
+from .audio_processing import is_flac, load_audio, load_audio_cuda, save_audio
 from .models import AudioDenoiser, AudioSuperResolution, StereoSeparator
 
 DEFAULT_CHUNK = 44100     # 2.0 s at 22.05 kHz (trainer.py:652)
@@ -535,16 +535,16 @@ def chunked_model_eval(model, waveform: torch.Tensor, chunk_size: int = 2 * 2205
 def generate_test_output(model, test_audio_dir: str, test_output_dir: str, suffix: str, device: str = "cuda",
                          max_seconds: int = 30) -> list:
     """Drop-in for `Trainer.generate_test_output` (src/training/trainer.py:582-721) as a free function: for every
-    `*.wav` in `test_audio_dir` (root only) take the first `max_seconds` of the mono 22.05 kHz signal, restore it in 2 s
-    chunks with `model`, and write `<stem>_original.wav` (once), `<stem>_degraded_<suffix>.wav` and
+    `*.wav` and `*.flac` in `test_audio_dir` (root only) take the first `max_seconds` of the mono 22.05 kHz signal, restore
+    it in 2 s chunks with `model`, and write `<stem>_original.wav` (once), `<stem>_degraded_<suffix>.wav` and
     `<stem>_restored_<suffix>.wav`; for `epoch_<k>` suffixes older epoch files of the same stem are deleted.
-    Returns the restored file paths.  (mp3/flac/ogg inputs of the reference need soundfile, which this image lacks.)"""
+    Returns the restored file paths.  (mp3/ogg inputs of the reference need soundfile.)"""
     import glob
     import os
     os.makedirs(test_output_dir, exist_ok=True)
     written = []
     model.eval()
-    for path in sorted(glob.glob(os.path.join(test_audio_dir, "*.wav"))):
+    for path in sorted(glob.glob(os.path.join(test_audio_dir, "*.wav")) + glob.glob(os.path.join(test_audio_dir, "*.flac"))):
         stem = os.path.splitext(os.path.basename(path))[0]
         original = os.path.join(test_output_dir, f"{stem}_original.wav")
         if not os.path.exists(original):
@@ -602,7 +602,7 @@ def restore_audio(
     print(f"Processing: {input_path}")
     print(f"Device: {device}")
     print("Loading audio...")
-    if input_path.lower().endswith(".wav"):
+    if input_path.lower().endswith(".wav") or is_flac(input_path):
         audio, _ = load_audio_cuda(input_path, sample_rate=sample_rate, device=device)   # decode / mono mix / resample on the GPU
     else:
         audio, _ = load_audio(input_path, sample_rate=sample_rate, mono=True)
