@@ -184,6 +184,28 @@ int ar_flac_decode(const uint8_t* frames, int64_t nbytes, int channels, int bps,
                    int64_t total_samples, float* y, int64_t n, int64_t* n_out, void* workspace, size_t workspace_bytes,
                    void* stream);
 
+/* FLAC output: torchaudio.save of a .flac path (audio_processing.py:45-55), encoded on the device (RFC 9639).
+ *   ar_flac_encode_workspace_bytes : device scratch (*workspace) and frame-output bytes (*out_capacity) ar_flac_encode needs
+ *                             for `channels` x `n` samples at `block_size` and `bps`; AR_ERR_INVALID for arguments
+ *                             ar_flac_encode rejects
+ *   ar_flac_encode          : x = planar fp32 [channels][n] (DEVICE), channels 1..8, bps 16 or 24, sample_rate 1..655350,
+ *                             block_size 16..4608 -> frames_out[out_capacity] (DEVICE) = the frame section of the stream
+ *                             (the caller writes `fLaC` and STREAMINFO in front: min = max block = block_size) and
+ *                             pcm_le_out (DEVICE, n * channels * bps / 8 bytes) = the interleaved little-endian samples
+ *                             the STREAMINFO MD5 is taken over.  Samples are rint_even(clamp(x, -1, 1) * (2^(bps-1) - 1))
+ *                             (fp32 multiply; NaN -> 0), as the pcm16 WAV writer rounds.  Fixed blocking (frame numbers,
+ *                             short last frame); per channel the fewest exact bits of CONSTANT, FIXED orders 0..4 (Rice /
+ *                             Rice2 and partition order searched exactly) and VERBATIM, with wasted bits; for two
+ *                             channels the cheapest of independent / left-side / side-right / mid-side.  The output is
+ *                             byte-identical to tests/flac_encode_ref.py::encode_search.  *frame_bytes_total, *min_frame,
+ *                             *max_frame receive the bytes of the frame section and of its smallest and largest frame.
+ *                             Synchronises `stream` once to read them.  A frame that did not write exactly the bits it
+ *                             was sized for returns AR_ERR_INVALID naming the frame. */
+int ar_flac_encode_workspace_bytes(int channels, int64_t n, int block_size, int bps, size_t* workspace, size_t* out_capacity);
+int ar_flac_encode(const float* x, int channels, int64_t n, int bps, int sample_rate, int block_size, uint8_t* frames_out,
+                   size_t out_capacity, uint8_t* pcm_le_out, int64_t* frame_bytes_total, int* min_frame, int* max_frame,
+                   void* workspace, size_t workspace_bytes, void* stream);
+
 /* Synthetic 78 rpm degradation generator (simulate_vinyl_artifacts, audio_processing.py:122-226; SURVEY.md 8f n4).
  * The random draws (np.random levels / pop plan, torch.randn noise tensors) stay with the caller; these entry points
  * are the deterministic arithmetic, rows = channels (or any batch of equal-length rows), all device fp32 [rows][n]:

@@ -58,6 +58,11 @@ _SIGNATURES = {
     "ar_flac_workspace_bytes": (C.c_int, [C.c_int64, C.POINTER(C.c_size_t)]),
     "ar_flac_decode": (C.c_int, [C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int64, C.c_void_p,
                                  C.c_int64, C.POINTER(C.c_int64), C.c_void_p, C.c_size_t, C.c_void_p]),
+    "ar_flac_encode_workspace_bytes": (C.c_int, [C.c_int, C.c_int64, C.c_int, C.c_int, C.POINTER(C.c_size_t),
+                                                 C.POINTER(C.c_size_t)]),
+    "ar_flac_encode": (C.c_int, [C.c_void_p, C.c_int, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p,
+                                 C.POINTER(C.c_int64), C.POINTER(C.c_int), C.POINTER(C.c_int), C.c_void_p, C.c_size_t,
+                                 C.c_void_p]),
     "ar_butter": (C.c_int, [C.c_int, C.c_double, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
     "ar_vinyl_mix": (C.c_int, [C.c_void_p, C.c_void_p, C.c_float, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int64,
                                C.c_void_p]),

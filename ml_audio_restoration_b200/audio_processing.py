@@ -1,13 +1,14 @@
 """Audio helpers on the restoration path (reference: src/utils/audio_processing.py).
 
 What inference needs -- `normalize_audio` (device kernel, no host syncs), `chunk_audio` (the reference's chunk
-vocabulary), small WAV load/save helpers and a GPU FLAC decoder so `restore_audio` works without `soundfile` --
+vocabulary), small WAV load/save helpers and a GPU FLAC decoder and encoder so `restore_audio` works without `soundfile` --
 plus the synthetic degradation generator `simulate_vinyl_artifacts` (SURVEY.md 8f n4) that produces the path's
 78 rpm-like inputs, with its pops and zero-phase Butterworth filters on the GPU.
 """
 from __future__ import annotations
 
 import ctypes as C
+import hashlib
 import wave
 
 import numpy as np
@@ -465,15 +466,74 @@ def load_audio_cuda(file_path: str, sample_rate: int = 22050, device="cuda"):
     return resample_mono_cuda(planar, sr, sample_rate), sample_rate
 
 
-def save_audio(file_path: str, audio: torch.Tensor, sample_rate: int = 22050, encoding: str = "float32") -> None:
-    """Write `[C,N]` float audio as WAV (audio_processing.py:45-55).  The reference's `torchaudio.save` of a float
-    tensor writes 32-bit IEEE-float samples; `encoding="pcm16"` writes 16-bit PCM instead."""
+def encode_flac_cuda(audio: torch.Tensor, sample_rate: int, bps: int = 24, block_size: int = 4096) -> bytes:
+    """Planar `[C, N]` (or `[N]`) float CUDA audio -> a complete .flac file (`fLaC`, STREAMINFO with the MD5, the frames),
+    encoded on the audio's device and current stream (`ar_flac_encode`).  Samples are
+    rint_even(clamp(x, -1, 1) * (2^(bps-1) - 1)), NaN -> 0, as `save_audio(..., encoding="pcm16")` rounds for WAV;
+    bps 16 or 24, 1..8 channels, block_size 16..4608.  The PCM bytes come back in pinned memory first and are hashed while
+    the frame bytes are still copying."""
+    if not audio.is_cuda:
+        raise RuntimeError("encode_flac_cuda: expected a CUDA tensor -- this build has no CPU fallback")
+    x = audio.detach().to(torch.float32)
+    x = (x[None] if x.dim() == 1 else x).contiguous()
+    if x.dim() != 2:
+        raise ValueError("encode_flac_cuda: expected [channels, samples] audio")
+    channels, n = x.shape
+    if not 1 <= int(sample_rate) <= 655350:
+        raise ValueError(f"encode_flac_cuda: sample rate {sample_rate} Hz (1..655350 supported)")
+    L = _lib.lib()
+    ws, cap = C.c_size_t(), C.c_size_t()
+    try:
+        _lib.check(L.ar_flac_encode_workspace_bytes(channels, n, int(block_size), int(bps), C.byref(ws), C.byref(cap)))
+    except RuntimeError as e:
+        raise ValueError(str(e)) from None
+    total, min_frame, max_frame = C.c_int64(), C.c_int(), C.c_int()
+    with torch.cuda.device(x.device):
+        stream = torch.cuda.current_stream(x.device)
+        work = torch.empty(ws.value, dtype=torch.uint8, device=x.device)
+        frames = torch.empty(cap.value, dtype=torch.uint8, device=x.device)
+        pcm = torch.empty(n * channels * (bps // 8), dtype=torch.uint8, device=x.device)
+        _lib.check(L.ar_flac_encode(x.data_ptr(), channels, n, int(bps), int(sample_rate), int(block_size), frames.data_ptr(),
+                                    cap.value, pcm.data_ptr(), C.byref(total), C.byref(min_frame), C.byref(max_frame),
+                                    work.data_ptr(), ws.value, stream.cuda_stream))
+        pcm_host = torch.empty(pcm.numel(), dtype=torch.uint8).pin_memory()
+        frames_host = torch.empty(total.value, dtype=torch.uint8).pin_memory()
+        pcm_host.copy_(pcm, non_blocking=True)
+        pcm_done = torch.cuda.Event()
+        pcm_done.record(stream)
+        frames_host.copy_(frames[:total.value], non_blocking=True)
+        pcm_done.synchronize()
+        md5 = hashlib.md5(pcm_host.numpy()).digest()
+        stream.synchronize()
+    info = int(sample_rate) << 44 | (channels - 1) << 41 | (bps - 1) << 36 | n
+    streaminfo = (int(block_size).to_bytes(2, "big") * 2 + min_frame.value.to_bytes(3, "big") + max_frame.value.to_bytes(3, "big")
+                  + info.to_bytes(8, "big") + md5)
+    return b"fLaC" + bytes([0x80]) + len(streaminfo).to_bytes(3, "big") + streaminfo + frames_host.numpy().tobytes()
+
+
+def save_audio(file_path: str, audio: torch.Tensor, sample_rate: int = 22050, encoding: str = None) -> None:
+    """Write `[C,N]` float audio (audio_processing.py:45-55), the container chosen by the extension as `torchaudio.save`
+    chooses it.  A `.flac` path (any case) writes FLAC encoded on the GPU (`encode_flac_cuda`): `encoding` "pcm24" (the
+    default) or "pcm16"; a CUDA tensor is encoded on its device, a host tensor on the current CUDA device.  Any other
+    path writes WAV: `encoding` None / "float32" writes 32-bit IEEE-float samples (what the reference's `torchaudio.save`
+    of a float tensor writes), "pcm16" / "pcm24" 16 / 24-bit PCM rounded as rint(clamp(x, -1, 1) * (2^(bits-1) - 1))."""
     import os
     import struct
+    parent = os.path.dirname(os.path.abspath(file_path))
+    if file_path.lower().endswith(".flac"):
+        encoding = "pcm24" if encoding is None else encoding
+        if encoding not in ("pcm16", "pcm24"):
+            raise ValueError(f"unknown FLAC encoding {encoding!r}: FLAC stores integers, use 'pcm16' or 'pcm24'")
+        x = audio.detach()
+        data = encode_flac_cuda(x if x.is_cuda else x.to(torch.device("cuda", torch.cuda.current_device())), sample_rate,
+                                bps=16 if encoding == "pcm16" else 24)
+        os.makedirs(parent, exist_ok=True)
+        with open(file_path, "wb") as f:
+            f.write(data)
+        return
     a = audio.detach().to("cpu", torch.float32).numpy()
     if a.ndim == 1:
         a = a[None]
-    parent = os.path.dirname(os.path.abspath(file_path))
     os.makedirs(parent, exist_ok=True)
     if encoding == "pcm16":
         pcm = np.round(np.clip(a, -1.0, 1.0).T * 32767.0).astype("<i2")
@@ -483,7 +543,16 @@ def save_audio(file_path: str, audio: torch.Tensor, sample_rate: int = 22050, en
             w.setframerate(int(sample_rate))
             w.writeframes(pcm.tobytes())
         return
-    if encoding != "float32":
+    if encoding == "pcm24":
+        v = np.ascontiguousarray(np.round(np.clip(np.nan_to_num(a, nan=0.0), -1.0, 1.0).T * np.float32(8388607.0)), "<i4")
+        pcm = v.view(np.uint8).reshape(-1, 4)[:, :3]                   # 3-byte little-endian samples
+        with wave.open(file_path, "wb") as w:
+            w.setnchannels(a.shape[0])
+            w.setsampwidth(3)
+            w.setframerate(int(sample_rate))
+            w.writeframes(pcm.tobytes())
+        return
+    if encoding not in (None, "float32"):
         raise ValueError(f"unknown WAV encoding {encoding!r}")
     data = np.ascontiguousarray(a.T).astype("<f4").tobytes()
     nch, sr = a.shape[0], int(sample_rate)

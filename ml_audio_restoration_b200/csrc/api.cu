@@ -23,6 +23,10 @@ int flac_workspace_bytes(long long nbytes, size_t* bytes);
 int flac_decode(const unsigned char* data, long long nbytes, int channels, int bps, int sample_rate, int min_block,
                 int max_block, long long total_samples, float* y, long long n, long long* n_out, void* ws, size_t ws_bytes,
                 cudaStream_t stream);
+int flac_encode_workspace_bytes(int channels, long long n, int block_size, int bps, size_t* workspace, size_t* out_capacity);
+int flac_encode(const float* x, int channels, long long n, int bps, int sample_rate, int block_size, unsigned char* frames_out,
+                size_t out_capacity, unsigned char* pcm_le_out, long long* frame_bytes_total, int* min_frame, int* max_frame,
+                void* ws, size_t ws_bytes, cudaStream_t stream);
 int butter(int order, double wn, int highpass, double* b, double* a);
 int launch_vinyl_mix(const float* audio, const float* noise, float level, const void* pops, int n_pops, int sample_rate,
                      float* y, int rows, long long n, cudaStream_t stream);
@@ -84,6 +88,18 @@ int ar_flac_decode(const uint8_t* frames, int64_t nbytes, int channels, int bps,
   const int rc = ar::flac_decode(frames, nbytes, channels, bps, sample_rate, min_block, max_block, total_samples, y, n, &got,
                                  workspace, workspace_bytes, reinterpret_cast<cudaStream_t>(stream));
   if (n_out) *n_out = got;
+  return rc;
+}
+int ar_flac_encode_workspace_bytes(int channels, int64_t n, int block_size, int bps, size_t* workspace, size_t* out_capacity) {
+  return ar::flac_encode_workspace_bytes(channels, n, block_size, bps, workspace, out_capacity);
+}
+int ar_flac_encode(const float* x, int channels, int64_t n, int bps, int sample_rate, int block_size, uint8_t* frames_out,
+                   size_t out_capacity, uint8_t* pcm_le_out, int64_t* frame_bytes_total, int* min_frame, int* max_frame,
+                   void* workspace, size_t workspace_bytes, void* stream) {
+  long long total = 0;
+  const int rc = ar::flac_encode(x, channels, n, bps, sample_rate, block_size, frames_out, out_capacity, pcm_le_out, &total,
+                                 min_frame, max_frame, workspace, workspace_bytes, reinterpret_cast<cudaStream_t>(stream));
+  if (frame_bytes_total) *frame_bytes_total = total;
   return rc;
 }
 int ar_butter(int order, double wn, int highpass, double* b, double* a) { return ar::butter(order, wn, highpass, b, a); }

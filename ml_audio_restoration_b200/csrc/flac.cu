@@ -24,6 +24,7 @@
 #include <vector>
 
 #include "ar_common.cuh"
+#include "flac_common.cuh"
 
 namespace ar {
 
@@ -68,15 +69,6 @@ struct FlacCand {        // one candidate frame (host copy of the table after th
 struct FlacChain {       // one frame of the chain: where it starts in the data and in the output
   long long off, first;
 };
-
-__host__ __device__ inline unsigned crc8_bytes(const unsigned char* p, int n) {
-  unsigned c = 0;
-  for (int i = 0; i < n; ++i) {
-    c ^= p[i];
-    for (int b = 0; b < 8; ++b) c = (c & 0x80) ? ((c << 1) ^ 0x07) & 0xFF : (c << 1) & 0xFF;
-  }
-  return c;
-}
 
 // Frame header at p[0..avail): fields resolved against STREAMINFO (codes 0 = "from STREAMINFO").
 __host__ __device__ inline int parse_header(const unsigned char* p, long long avail, const StreamParams& sp, FlacHeader* h) {
@@ -465,15 +457,6 @@ __global__ void __launch_bounds__(INDEX_THREADS) flac_compact_kernel(const unsig
     }
     ++at;
   }
-}
-
-__device__ void crc16_table(unsigned short* tab) {
-  for (int v = threadIdx.x; v < 256; v += blockDim.x) {
-    unsigned c = (unsigned)v << 8;
-    for (int b = 0; b < 8; ++b) c = (c & 0x8000) ? ((c << 1) ^ 0x8005) & 0xFFFF : (c << 1) & 0xFFFF;
-    tab[v] = (unsigned short)c;
-  }
-  __syncthreads();
 }
 
 __global__ void __launch_bounds__(FT) flac_walk_kernel(const unsigned char* __restrict__ data, long long nbytes, StreamParams sp,

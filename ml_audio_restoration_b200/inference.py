@@ -590,12 +590,15 @@ def restore_audio(
     mode: str = 'whole',
     chunk_size: int = DEFAULT_CHUNK,
     overlap: int = DEFAULT_OVERLAP,
+    output_encoding: str = None,
 ):
     """Drop-in for the reference `restore_audio` (inference.py:17-108): same positional/keyword
-    arguments and progress prints; `mode`, `chunk_size`, `overlap` are additions (default
+    arguments and progress prints; `mode`, `chunk_size`, `overlap`, `output_encoding` are additions (default
     `mode='whole'` keeps the reference's whole-file semantics; `'chunked'` is the fast path, `'exact'` the
     bounded-memory chunked form of `'whole'`).  Before restoring, the checkpoints' dynamic range is audited on a few
-    chunks of the file (`RestorationPipeline.check_dynamic_range`).
+    chunks of the file (`RestorationPipeline.check_dynamic_range`).  The output container follows the extension of
+    `output_path` (`save_audio`): a `.flac` path is encoded on the GPU straight from the restored device tensor;
+    `output_encoding` ("float32" for WAV only, "pcm16", "pcm24") defaults to float32 WAV / 24-bit FLAC.
     """
     if torch.device(device).type != 'cuda':
         raise RuntimeError("restore_audio: device must be a CUDA device -- this build has no CPU fallback")
@@ -624,7 +627,7 @@ def restore_audio(
     stereo = pipe.restore(audio, mode=mode, chunk_size=chunk_size, overlap=overlap)
     out_rate = sample_rate * pipe.rate
     print(f"Saving to: {output_path}")
-    save_audio(output_path, stereo, out_rate)
+    save_audio(output_path, stereo, out_rate, encoding=output_encoding)
     print("Restoration complete!")
     suffix = " (bandwidth extended)" if enable_super_resolution else ""
     print(f"Output sample rate: {out_rate}Hz{suffix}")
@@ -648,11 +651,13 @@ def main(argv=None):
                          "'exact' = chunked with conv halos and LSTM state carry, equal to 'whole' in bounded memory")
     ap.add_argument('--chunk-size', type=int, default=DEFAULT_CHUNK)
     ap.add_argument('--overlap', type=int, default=DEFAULT_OVERLAP)
+    ap.add_argument('--output-encoding', choices=('float32', 'pcm16', 'pcm24'), default=None,
+                    help="sample encoding of the output file (default: float32 for WAV, pcm24 for FLAC; FLAC stores integers)")
     a = ap.parse_args(argv)
     restore_audio(a.input, a.output, denoiser_checkpoint=a.denoiser, super_res_checkpoint=a.super_res,
                   stereo_checkpoint=a.stereo, sample_rate=a.sample_rate,
                   enable_super_resolution=not a.no_super_res, device=a.device, mode=a.mode,
-                  chunk_size=a.chunk_size, overlap=a.overlap)
+                  chunk_size=a.chunk_size, overlap=a.overlap, output_encoding=a.output_encoding)
 
 
 if __name__ == "__main__":
