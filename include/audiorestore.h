@@ -107,6 +107,11 @@ int ar_model_forward(ar_model_t m, const float* x, float* y, int B, int T,
 int ar_model_audit_enable(ar_model_t m, int on);
 int ar_model_audit_read(ar_model_t m, float* max_abs, int cap, int* n_layers);
 const char* ar_model_audit_name(ar_model_t m, int i);
+/* Test hook on the audit path: while the audit is on, every forward that writes the audited tensor `name` also copies the
+ * channel window it wrote into the device buffer y as plain fp32 [B][channels][T] (rows [0,T) only).  Several names may be
+ * armed at once; arming a name again replaces its buffer; a NULL name disarms all.  A window of more than cap_floats
+ * values makes that forward return AR_ERR_INVALID before the copy is launched.  Forwards with the audit off ignore taps. */
+int ar_model_audit_tap(ar_model_t m, const char* name, float* y, int64_t cap_floats);
 
 /* Stereo forward with explicit LSTM carry (whole-file-exact mode, SURVEY.md 8 n2):
  * state_in/state_out are [B,2,64] (h then c) device buffers; either may be NULL. */

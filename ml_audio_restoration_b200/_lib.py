@@ -40,6 +40,7 @@ _SIGNATURES = {
     "ar_model_audit_enable": (C.c_int, [C.c_void_p, C.c_int]),
     "ar_model_audit_read": (C.c_int, [C.c_void_p, C.POINTER(C.c_float), C.c_int, C.POINTER(C.c_int)]),
     "ar_model_audit_name": (C.c_char_p, [C.c_void_p, C.c_int]),
+    "ar_model_audit_tap": (C.c_int, [C.c_void_p, C.c_char_p, C.c_void_p, C.c_int64]),
     "ar_model_workspace_bytes": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_size_t)]),
     "ar_model_forward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p]),
     "ar_stereo_forward_state": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p,

@@ -46,6 +46,7 @@ int model_kind(const Model* m);
 int model_audit_enable(Model* m, int on);
 int model_audit_read(Model* m, float* max_abs, int cap, int* n_layers);
 const char* model_audit_name(const Model* m, int i);
+int model_audit_tap(Model* m, const char* name, float* y, long long cap_floats);
 struct ConvLayerPublic;
 int debug_conv(const float* x, const float* w_host, const float* bias_host, float* y, int B, int Cin, int Cout, int T, int k,
                int dil, int lrelu, int engine, cudaStream_t stream);
@@ -136,6 +137,9 @@ int ar_model_audit_read(ar_model_t m, float* max_abs, int cap, int* n_layers) {
   return ar::model_audit_read(reinterpret_cast<ar::Model*>(m), max_abs, cap, n_layers);
 }
 const char* ar_model_audit_name(ar_model_t m, int i) { return ar::model_audit_name(reinterpret_cast<ar::Model*>(m), i); }
+int ar_model_audit_tap(ar_model_t m, const char* name, float* y, int64_t cap_floats) {
+  return ar::model_audit_tap(reinterpret_cast<ar::Model*>(m), name, y, cap_floats);
+}
 
 int ar_model_workspace_bytes(ar_model_t m, int B, int T, size_t* bytes) {
   return ar::model_workspace_bytes(reinterpret_cast<ar::Model*>(m), B, T, bytes);

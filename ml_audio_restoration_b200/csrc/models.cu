@@ -203,6 +203,8 @@ struct Model {
   bool audit = false;
   unsigned int* audit_dev = nullptr;
   std::vector<std::string> audit_names;
+  struct Tap { float* y; long long cap; };
+  std::map<std::string, Tap> audit_taps;   // ar_model_audit_tap: audited tensors also copied out as plain fp32
   ~Model() { if (blob) cudaFree(blob); if (audit_dev) cudaFree(audit_dev); }
 };
 constexpr int AUDIT_SLOTS = AR_AUDIT_MAX_LAYERS;
@@ -564,6 +566,13 @@ static int audit_act(Ctx& c, const std::string& name, const Act& a, int coff8, i
   if (slot == m->audit_names.size()) {
     AR_CHECK(slot < (size_t)AUDIT_SLOTS, AR_ERR_INVALID, "internal: too many audited layers");
     m->audit_names.push_back(name);
+  }
+  auto tap = m->audit_taps.find(name);
+  if (tap != m->audit_taps.end()) {
+    const long long n = (long long)c.B * nch8 * 8 * T;
+    AR_CHECK(n <= tap->second.cap, AR_ERR_INVALID,
+             "audit tap " + name + ": window of " + std::to_string(n) + " floats exceeds the buffer (" + std::to_string(tap->second.cap) + ")");
+    AR_TRY(launch_audit_tap(a, c.B, coff8, nch8, T, tblock, tap->second.y, c.stream));
   }
   return launch_audit(a, c.B, coff8, nch8, T, tblock, m->audit_dev + slot, c.stream);
 }
@@ -966,6 +975,7 @@ static int stereo_forward(Ctx& c, const float* x, float* y, int T, const float* 
   AR_TRY(stereo_encode(c, x, T, xp, fp));
   Act h = A.act(c.B, 64, T);
   AR_TRY(stereo_scan(c, xp, h, T, state_in, state_out, w, fp));
+  AR_TRY(audit_act(c, "lstm", h, 0, 64 / 8, T));
   A.release(xp);
   return stereo_decode(c, h, y, T, true);
 }
@@ -1129,6 +1139,13 @@ int model_audit_read(Model* m, float* max_abs, int cap, int* n_layers) {
 }
 const char* model_audit_name(const Model* m, int i) {
   return (m && i >= 0 && i < (int)m->audit_names.size()) ? m->audit_names[i].c_str() : nullptr;
+}
+int model_audit_tap(Model* m, const char* name, float* y, long long cap_floats) {
+  AR_CHECK(m != nullptr, AR_ERR_INVALID, "audit tap: null model");
+  if (name == nullptr) { m->audit_taps.clear(); return AR_OK; }
+  AR_CHECK(y != nullptr && cap_floats >= 0, AR_ERR_INVALID, "audit tap: null buffer or negative capacity");
+  m->audit_taps[name] = Model::Tap{y, cap_floats};
+  return AR_OK;
 }
 
 void model_destroy(Model* m) { delete m; }

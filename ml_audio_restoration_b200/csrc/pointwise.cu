@@ -513,12 +513,16 @@ __global__ void plain_to_h8_kernel(const float* __restrict__ x, int C, int T, __
   for (int i = 0; i < 8; ++i) v[i] = x[((long long)b * C + c8 * 8 + i) * T + t];
   *reinterpret_cast<uint4*>(out + act_off(bs, Tp, b, c8, t)) = pack_half8(v);
 }
-__global__ void h8_to_plain_kernel(const __half* __restrict__ in, long long bs, int Tp, int C, int T, float* __restrict__ y) {
+// channel chunks [coff8, coff8 + gridDim.y) of an H8 (or, with tblock, time-blocked H8 of C8 chunks) tensor -> plain fp32
+// [B][C][T] with C = 8 * gridDim.y
+__global__ void h8_to_plain_kernel(const __half* __restrict__ in, long long bs, int Tp, int C8, int coff8, int tblock, int C, int T,
+                                   float* __restrict__ y) {
   const int b = blockIdx.z, c8 = blockIdx.y;
   const int t = blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= T) return;
+  const long long off = tblock ? act_off_tb(bs, C8, b, coff8 + c8, t) : act_off(bs, Tp, b, coff8 + c8, t);
   float v[8];
-  unpack_half8(*reinterpret_cast<const uint4*>(in + act_off(bs, Tp, b, c8, t)), v);
+  unpack_half8(*reinterpret_cast<const uint4*>(in + off), v);
   for (int i = 0; i < 8; ++i) y[((long long)b * C + c8 * 8 + i) * T + t] = v[i];
 }
 int launch_plain_to_c4(const float* x, int B, int C, int T, const Act& out, cudaStream_t stream) {
@@ -529,7 +533,13 @@ int launch_plain_to_c4(const float* x, int B, int C, int T, const Act& out, cuda
 }
 int launch_c4_to_plain(const Act& in, int B, int C, int T, float* y, cudaStream_t stream) {
   dim3 grid((T + 127) / 128, C / 8, B);
-  h8_to_plain_kernel<<<grid, 128, 0, stream>>>(in.h(), in.bs, in.Tp, C, T, y);
+  h8_to_plain_kernel<<<grid, 128, 0, stream>>>(in.h(), in.bs, in.Tp, in.C / 8, 0, 0, C, T, y);
+  AR_CUDA_OK(cudaGetLastError());
+  return AR_OK;
+}
+int launch_audit_tap(const Act& a, int B, int coff8, int nch8, int T, int tblock, float* y, cudaStream_t stream) {
+  dim3 grid((T + 127) / 128, nch8, B);
+  h8_to_plain_kernel<<<grid, 128, 0, stream>>>(a.h(), a.bs, a.Tp, a.C / 8, coff8, tblock, nch8 * 8, T, y);
   AR_CUDA_OK(cudaGetLastError());
   return AR_OK;
 }

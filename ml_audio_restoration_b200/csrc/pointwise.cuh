@@ -44,6 +44,8 @@ int launch_ola(const float* y, float* out, long long n, int n_chunks, int channe
 // max |value| over rows [0,T) of channel chunks [coff8, coff8 + nch8) of an activation tensor -> atomic max into *slot
 // (float bits); dynamic-range audit
 int launch_audit(const Act& a, int B, int coff8, int nch8, int T, int tblock, unsigned int* slot, cudaStream_t stream);
+// the same window as plain fp32 [B][8 nch8][T] (ar_model_audit_tap)
+int launch_audit_tap(const Act& a, int B, int coff8, int nch8, int T, int tblock, float* y, cudaStream_t stream);
 int launch_plain_to_c4(const float* x, int B, int C, int T, const Act& out, cudaStream_t stream);
 int launch_c4_to_plain(const Act& in, int B, int C, int T, float* y, cudaStream_t stream);
 

@@ -59,3 +59,28 @@ def debug_conv(x, w, b, dilation=1, lrelu=0, engine=_lib.ENGINE_UMMA):
     _lib.check(_lib.lib().ar_debug_conv1d(xc.data_ptr(), wc.data_ptr(), bc.data_ptr(), y.data_ptr(), B, Cin, Cout, T, k,
                                           dilation, lrelu, engine, torch.cuda.current_stream().cuda_stream))
     return y.cpu()
+
+
+def audit_taps(module, x, shapes):
+    """Run `module`'s forward on x under the dynamic-range audit (layer by layer) with every tensor of `shapes`
+    ({name: (channels, length)}) tapped through `ar_model_audit_tap`.  Returns ({name: fp32 [B, C, T] device tensor}, y,
+    {name: max |value|}).  Tap buffers start as NaN, so a window the forward did not copy in full cannot pass a check."""
+    x = module._check_input(x)
+    B = x.shape[0]
+    L = _lib.lib()
+    taps = {n: torch.full((B, c, t), float("nan"), device=x.device) for n, (c, t) in shapes.items()}
+    with torch.cuda.device(x.device):
+        h = module.native_handle(x.device)
+        for n, buf in taps.items():
+            _lib.check(L.ar_model_audit_tap(h, n.encode(), buf.data_ptr(), buf.numel()))
+        _lib.check(L.ar_model_audit_enable(h, 1))
+        try:
+            y = module.forward(x)
+            vals = (C.c_float * _lib.AUDIT_MAX_LAYERS)()
+            n = C.c_int()
+            _lib.check(L.ar_model_audit_read(h, vals, _lib.AUDIT_MAX_LAYERS, C.byref(n)))
+            audit = {L.ar_model_audit_name(h, i).decode(): float(vals[i]) for i in range(n.value)}
+        finally:
+            L.ar_model_audit_enable(h, 0)
+            L.ar_model_audit_tap(h, None, None, 0)
+    return taps, y, audit

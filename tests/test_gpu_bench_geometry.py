@@ -8,8 +8,8 @@ import torch
 
 import oracle
 from oracle import pipeline as opipe
-from oracle.models import calibrate_batchnorm, stereo_forward_window
-from oracle.weights import make_input, make_state_dict
+from oracle.models import stereo_forward_window
+from oracle.weights import calibrated_state_dicts, make_input, make_state_dict
 from ml_audio_restoration_b200 import RestorationPipeline
 from gpu_util import make_model, assert_close
 
@@ -117,28 +117,41 @@ def test_config4_full_side_vs_oracle(pipe, state_dicts):
     assert_close(ref, y, "config 4: 180 s side, 95 chunks, normalize on, vs oracle")
 
 
-@pytest.mark.parametrize("fusion", [1, 0], ids=["projection-in-scan", "stored-pre-activations"])
-def test_stereo_beyond_eight_per_sm_every_sequence_vs_oracle(state_dicts, fusion):
+@pytest.fixture(scope="module")
+def calibrated():
+    return calibrated_state_dicts()
+
+
+@pytest.mark.parametrize("fusion,weights", [(1, "benign"), (0, "benign"), (1, "calibrated")],
+                         ids=["projection-in-scan", "stored-pre-activations", "projection-in-scan-calibrated"])
+def test_stereo_beyond_eight_per_sm_every_sequence_vs_oracle(state_dicts, calibrated, fusion, weights):
     """More than 8 sequences per SM: the scan kernel that computes the LSTM input projection itself (`lstm_proj_kernel`:
     tcgen05 GEMM per 8-step block + two 8-sequence recurrence groups per CTA; product path) and, layer by layer,
     `lstm_mmaw_kernel<8>` on stored pre-activations (cross-check path).  EVERY sequence of a ragged batch (1197 = 74 full
-    CTAs of 16 + 13 sequences) and ragged length (203 = 25 blocks + 3 steps) against the oracle, outputs and final (h, c);
-    the two paths against each other (same fp16 pre-activations => the same recurrence)."""
-    m = make_model("stereo", state_dicts["stereo"], fusion=fusion)
+    CTAs of 16 + 13 sequences) and ragged length (203 = 25 blocks + 3 steps) against the oracle, outputs and final (h, c)
+    (benign weights); the two paths against each other, bitwise (same fp16 pre-activations => the same recurrence), with
+    both weight sets -- with calibrated ones the layer-by-layer path is pinned layer by layer (test_gpu_layers.py)."""
+    sd = state_dicts["stereo"] if weights == "benign" else calibrated["stereo"]
+    m = make_model("stereo", sd, fusion=fusion)
     B, T = huge_batch(), 203
     x = make_input(B, T, seed=37)
-    ref, (hn, cn) = oracle.stereo_forward(state_dicts["stereo"], x, return_state=True)
     with torch.no_grad():
         y, st = m.forward_with_state(x.cuda())
-    assert_close(ref, y, f"stereo B={B} T={T} (beyond 8 sequences per SM, fusion={fusion})")
-    assert_close(hn[0], st[:, 0], "carried h", max_abs=1e-3, min_snr=50.0)
-    assert_close(cn[0], st[:, 1], "carried c", max_abs=1e-3, min_snr=50.0)
+    if weights == "benign":
+        ref, (hn, cn) = oracle.stereo_forward(sd, x, return_state=True)
+        assert_close(ref, y, f"stereo B={B} T={T} (beyond 8 sequences per SM, fusion={fusion})")
+        assert_close(hn[0], st[:, 0], "carried h", max_abs=1e-3, min_snr=50.0)
+        assert_close(cn[0], st[:, 1], "carried c", max_abs=1e-3, min_snr=50.0)
+    else:
+        assert torch.isfinite(y).all() and torch.isfinite(st).all()
     if fusion == 1:
-        other = make_model("stereo", state_dicts["stereo"], fusion=0)
+        other = make_model("stereo", sd, fusion=0)
         with torch.no_grad():
             y0, st0 = other.forward_with_state(x.cuda())
-        assert_close(y0, y, "projection inside the scan vs stored pre-activations", max_abs=2e-5, min_snr=90.0)
-        assert_close(st0, st, "final states, projection inside the scan vs stored pre-activations", max_abs=2e-5, min_snr=90.0)
+        print(f"[{weights}] projection inside the scan vs stored pre-activations: max|diff| {float((y0 - y).abs().max()):.3e}, "
+              f"bitwise equal: outputs {torch.equal(y0, y)}, states {torch.equal(st0, st)}")
+        assert torch.equal(y0, y), "projection inside the scan vs stored pre-activations: outputs differ"
+        assert torch.equal(st0, st), "projection inside the scan vs stored pre-activations: final states differ"
 
 
 @pytest.mark.parametrize("T", [1, 5, 8, 9, 16, 17, 24])
@@ -244,19 +257,6 @@ def test_exact_mode_equals_whole_file_and_reference_golden(pipe, state_dicts, go
 
 
 # ------------------------------------------------------------------------------------------------ dynamic range
-def calibrated_state_dicts():
-    """Trained-like checkpoints: BatchNorm running stats = statistics of each layer's input on a calibration batch, so
-    running_var is as small as 1e-4 and the BN folds carry gains of up to ~100 per layer (oracle.calibrate_batchnorm)."""
-    x = make_input(4, 8192, 5)
-    sds, y = {}, x
-    sds["denoiser"], _ = calibrate_batchnorm("denoiser", make_state_dict("denoiser"), y)
-    y = oracle.denoiser_forward(sds["denoiser"], y)
-    sds["super_resolution"], _ = calibrate_batchnorm("super_resolution", make_state_dict("super_resolution"), y)
-    y = oracle.super_resolution_forward(sds["super_resolution"], y)
-    sds["stereo"], stats = calibrate_batchnorm("stereo", make_state_dict("stereo"), y)
-    return sds
-
-
 def torch_eager_tf32_chain(sds, x):
     """The reference's op sequence under stock torch eager on the GPU with TF32 allowed -- PyTorch's DEFAULT for cuDNN
     convolutions (`torch.backends.cudnn.allow_tf32 = True`), i.e. what `python src/inference.py --device cuda` computes."""
@@ -277,17 +277,17 @@ def torch_eager_tf32_chain(sds, x):
         torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32 = old
 
 
-def test_dynamic_range_full_scale_input_and_calibrated_batchnorm():
+def test_dynamic_range_full_scale_input_and_calibrated_batchnorm(calibrated):
     """The envelope of the 11-bit-significand operand path (fp16 storage == TF32 precision), with trained-like weights.
 
     Setting: (i) BatchNorm-calibrated checkpoints (folded gains up to ~100, activations at unit scale in every layer) and
     (ii) a full-scale input: pops that drive normalize_audio into its peak-limit branch (max |x| = 1.0).
-    Range: finite output and an audited headroom of more than 30x below the fp16 limit in every one of the 48 stored tensors.
+    Range: finite output and an audited headroom of more than 30x below the fp16 limit in every one of the 49 stored tensors.
     Precision: with unit-scale activations in ~50 layers, 11-bit operands cost more than with the near-degenerate random-init
     weights of the parity tests (81 dB there): ~42 dB against the fp32 oracle (CPU emulation of operand rounding alone gives
     41-43 dB).  That is the precision class of the reference's OWN GPU path -- PyTorch runs cuDNN convolutions in TF32 by
     default -- so the assertion is: not worse than torch-eager-TF32 on the same GPU by more than 3 dB, and >= 38 dB."""
-    sds = calibrated_state_dicts()
+    sds = calibrated
     pipe = RestorationPipeline.from_state_dicts(sds["denoiser"], sds["super_resolution"], sds["stereo"], "cuda")
     N = 3 * 8192
     audio = make_input(1, N, 9, scale=0.02)[0]
