@@ -65,17 +65,9 @@ int ar_set_conv_engine(int engine);
 /* Fused multi-layer launches (the StereoSeparator's dilated block conv k3 -> conv k1 [-> LSTM input projection],
  * stereo_separator.py:49-64,104-106, and the U-Net's / residual blocks' conv k3 -> conv k3 pairs, denoiser.py:51-60,
  * super_resolution.py:104-122, as one kernel whose intermediates stay in shared memory) for subsequently created
- * models: 0 = layer by layer, 1 (default) = the chains that measured faster than their layers, 2 = every chain that
- * fits.  Cross-check knob: all settings compute the same fp16-rounded intermediates. */
-int ar_set_fusion(int level);
-
-/* Shared memory one conv CTA may use, in KB (64..227, default 227 = the whole SM).  AR_CORESIDENT_SMEM_KB leaves room
- * for one CTA of the LSTM recurrence on every SM: when chunk batches are pipelined on two streams the latency-bound
- * scan of one batch (stereo_separator.py:106) then runs UNDER the convs of the other instead of after them (measured:
- * no gain on power-capped B200s, profiles/README_r01.md; kept as a tuning hook).
- * Takes effect for subsequent forwards (process-wide, like ar_set_conv_engine). */
-#define AR_CORESIDENT_SMEM_KB 172
-int ar_set_conv_smem_kb(int kb);
+ * models: 0 = layer by layer, 1 (default) = every chain that fits; anything else is AR_ERR_INVALID.  Cross-check knob:
+ * both settings compute the same fp16-rounded intermediates. */
+int ar_set_fusion(int on);
 
 /* Replaces: model construction + torch.load + load_state_dict(strict) + .to(device) + .eval()
  * (inference.py:51-55, 66-70, 85-89).  Folds eval-mode BatchNorm into the conv weights,

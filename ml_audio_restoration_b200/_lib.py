@@ -18,7 +18,6 @@ AR_OK, AR_ERR_INVALID, AR_ERR_WEIGHTS, AR_ERR_CUDA, AR_ERR_WORKSPACE = 0, 1, 2, 
 MODEL_DENOISER, MODEL_SUPER_RES, MODEL_STEREO = 0, 1, 2
 ENGINE_UMMA, ENGINE_SIMT = 0, 1
 NORMALIZE_SCRATCH_BYTES = 16384
-CORESIDENT_SMEM_KB, FULL_SMEM_KB = 172, 227
 AUDIT_MAX_LAYERS = 64
 HALF_MAX = 65504.0
 PROFILE_CATEGORIES = ("conv", "lstm", "stem", "tail", "normalize", "chunk")
@@ -33,7 +32,6 @@ _SIGNATURES = {
     "ar_version": (C.c_int, []),
     "ar_set_conv_engine": (C.c_int, [C.c_int]),
     "ar_set_fusion": (C.c_int, [C.c_int]),
-    "ar_set_conv_smem_kb": (C.c_int, [C.c_int]),
     "ar_model_create": (C.c_int, [C.c_int, C.POINTER(ArTensor), C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     "ar_model_destroy": (None, [C.c_void_p]),
     "ar_model_kind": (C.c_int, [C.c_void_p]),

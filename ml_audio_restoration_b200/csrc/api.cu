@@ -47,7 +47,6 @@ int model_audit_enable(Model* m, int on);
 int model_audit_read(Model* m, float* max_abs, int cap, int* n_layers);
 const char* model_audit_name(const Model* m, int i);
 int model_audit_tap(Model* m, const char* name, float* y, long long cap_floats);
-struct ConvLayerPublic;
 int debug_conv(const float* x, const float* w_host, const float* bias_host, float* y, int B, int Cin, int Cout, int T, int k,
                int dil, int lrelu, int engine, cudaStream_t stream);
 }  // namespace ar
@@ -65,8 +64,7 @@ extern "C" {
 const char* ar_last_error(void) { return ar::last_error(); }
 int ar_version(void) { return 100; }
 int ar_set_conv_engine(int engine) { return ar::set_engine(engine); }
-int ar_set_fusion(int level) { return ar::set_fusion(level); }
-int ar_set_conv_smem_kb(int kb) { return ar::set_conv_smem_kb(kb); }
+int ar_set_fusion(int on) { return ar::set_fusion(on); }
 int ar_resample_length(int64_t n, int orig_sr, int new_sr, int64_t* n_out) {
   if (!n_out || n < 0 || orig_sr < 1 || new_sr < 1) { ar::set_error("resample_length: bad argument"); return AR_ERR_INVALID; }
   *n_out = ar::resample_length(n, orig_sr, new_sr);

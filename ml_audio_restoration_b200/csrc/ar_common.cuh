@@ -217,9 +217,5 @@ struct DeviceOnce {
   bool pending() const;
   void done();
 };
-// Shared memory a conv CTA may take (bytes): 227 KB by default (one CTA owns the SM); ar_set_conv_smem_kb lowers it so
-// that a CTA of the latency-bound LSTM recurrence can be co-resident on the same SM.
-int conv_smem_budget();
-int set_conv_smem_kb(int kb);
 
 }  // namespace ar

@@ -609,7 +609,7 @@ static bool pick_chain_cfg(const ChainParams& cp, ChainCfg& c) {
           off += c.nbI[g] * c.i_bytes[g];
         }
         c.stage_off = off;
-        const int room = conv_smem_budget() - CH_BAR_BYTES - CH_BIAS_BYTES - off;
+        const int room = CH_SMEM_BUDGET - CH_BAR_BYTES - CH_BIAS_BYTES - off;
         c.kbs = kbs;
         c.stage_bytes = kbs * 2 * c.R * 16;
         int stages = room / c.stage_bytes;

@@ -326,7 +326,7 @@ static bool pick_cfg2(const ConvParams& p, Umma2Cfg& c) {
   while (ncol < Ns) ncol <<= 1;
   c.ncol = ncol;
   c.w_bytes = p.Cin * p.taps * (Ns / 2) * 2;
-  const int room0 = conv_smem_budget() - BAR2_BYTES - BIAS2_BYTES - c.w_bytes;
+  const int room0 = SMEM2_BUDGET - BAR2_BYTES - BIAS2_BYTES - c.w_bytes;
   for (int kbs = 4; kbs >= 1; kbs >>= 1) {
     if (p.Cin % (16 * kbs)) continue;
     // group size: enough tiles per barrier round that a stage carries >= ~64 MMAs, within TMEM (two buffers) and the ring

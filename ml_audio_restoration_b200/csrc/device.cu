@@ -1,4 +1,4 @@
-// Per-device host state shared by the launchers: SM count, one-time kernel attributes, the conv shared-memory budget.
+// Per-device host state shared by the launchers: SM count and one-time kernel attributes.
 // Function attributes (cudaFuncSetAttribute) and the SM count belong to a device / context, not to the process: one
 // process may drive several GPUs (RestorationPipeline(device="cuda:1") next to "cuda:0"), so every "done once" flag here
 // is kept per device.
@@ -34,13 +34,5 @@ int sm_count() {
   }
   return v;
 }
-
-static std::atomic<int> g_conv_smem{227 * 1024};
-int set_conv_smem_kb(int kb) {
-  if (kb < 64 || kb > 227) { set_error("conv shared-memory budget must be within [64, 227] KB"); return AR_ERR_INVALID; }
-  g_conv_smem.store(kb * 1024);
-  return AR_OK;
-}
-int conv_smem_budget() { return g_conv_smem.load(); }
 
 }  // namespace ar

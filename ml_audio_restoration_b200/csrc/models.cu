@@ -26,12 +26,12 @@ int set_engine(int e) {
   g_engine.store(e);
   return AR_OK;
 }
-// Fused multi-layer launches (conv_chain.cu) for subsequently created models: 0 = layer by layer, 1 = the chains that
-// measured faster than their layers (product default), 2 = every chain that fits (parity cross-check of the k3 -> k3 kernels)
-static std::atomic<int> g_fuse{1};
-int set_fusion(int level) {
-  if (level < 0 || level > 2) { set_error("fusion level must be 0, 1 or 2"); return AR_ERR_INVALID; }
-  g_fuse.store(level);
+// Fused multi-layer launches (conv_chain.cu) for subsequently created models: 0 = layer by layer, 1 = every chain that
+// fits (product default)
+static std::atomic<bool> g_fuse{true};
+int set_fusion(int on) {
+  if (on != 0 && on != 1) { set_error("fusion must be 0 (layer by layer) or 1 (fused)"); return AR_ERR_INVALID; }
+  g_fuse.store(on == 1);
   return AR_OK;
 }
 static std::atomic<long long*> g_chain_trace{nullptr};   // debug: device buffer the fused-chain kernels trace their pipeline into
@@ -105,6 +105,11 @@ struct Blob {
     return off;
   }
   size_t push(const std::vector<float>& v) { return push(v.data(), v.size()); }
+  size_t push_half(const std::vector<uint16_t>& h) {   // a packed fp16 operand, zero-padded to whole floats
+    std::vector<float> raw((h.size() + 1) / 2);
+    std::memcpy(raw.data(), h.data(), h.size() * 2);
+    return push(raw);
+  }
   ConvLayer push_gemm(Gemm& g) {  // fp16 [n_slices][Cin/16][taps][2][Ns][8]
     const bool cta2 = want_cta2(g.N);
     // per-CTA slices: for the 2-CTA engine split every pair-slice once more (the budget applies per CTA)
@@ -129,9 +134,7 @@ struct Blob {
     }
     if (!(lmax <= w_max)) w_max = lmax;
     if (lmax < w_min_layer_max) w_min_layer_max = lmax;
-    std::vector<float> raw((w.size() + 1) / 2);
-    std::memcpy(raw.data(), w.data(), w.size() * 2);
-    L.w_off = push(raw);
+    L.w_off = push_half(w);
     L.b_off = push(g.bias);
     return L;
   }
@@ -187,7 +190,7 @@ static bool make_conv(const Table& t, Blob& blob, const std::string& conv, const
 
 struct Model {
   int kind = -1, device = 0, engine = AR_ENGINE_UMMA;
-  int fuse = 1;   // fused conv chains (tcgen05 engine, 2-CTA packing): 0 none, 1 measured-faster ones, 2 all that fit
+  bool fuse = true;   // fused conv chains (tcgen05 engine, 2-CTA packing) wherever the chain kernel takes the layers
   float* blob = nullptr;
   std::map<std::string, ConvLayer> conv;
   StemP stem{};          // Cin = 1 stem: kernel-parameter weights
@@ -209,8 +212,7 @@ struct Model {
 };
 constexpr int AUDIT_SLOTS = AR_AUDIT_MAX_LAYERS;
 
-static bool stem_pack(const Table& t, Blob& blob, const std::string& conv, const std::string& bn, int k, StemP& s) {
-  (void)blob;
+static bool stem_pack(const Table& t, const std::string& conv, const std::string& bn, int k, StemP& s) {
   const float* W = t.get(conv + ".weight", {32, 1, k});
   Fold f;
   if (!W || !fold_bn(t, conv, bn, 32, f)) return false;
@@ -225,7 +227,7 @@ static bool stem_pack(const Table& t, Blob& blob, const std::string& conv, const
 
 static bool build_denoiser(const Table& t, Blob& blob, Model& m) {
   const int F[3] = {32, 64, 128};
-  if (!stem_pack(t, blob, "encoder.0.0", "encoder.0.1", 3, m.stem)) return false;
+  if (!stem_pack(t, "encoder.0.0", "encoder.0.1", 3, m.stem)) return false;
   if (!make_conv(t, blob, "encoder.0.3", "encoder.0.4", 32, 32, 3, 1, m.conv["enc0b"])) return false;
   if (!make_conv(t, blob, "encoder.1.0", "encoder.1.1", 32, 64, 3, 1, m.conv["enc1a"])) return false;
   if (!make_conv(t, blob, "encoder.1.3", "encoder.1.4", 64, 64, 3, 1, m.conv["enc1b"])) return false;
@@ -283,7 +285,7 @@ static bool build_denoiser(const Table& t, Blob& blob, Model& m) {
 }
 
 static bool build_sr(const Table& t, Blob& blob, Model& m) {
-  if (!stem_pack(t, blob, "initial.0", "", 7, m.stem)) return false;
+  if (!stem_pack(t, "initial.0", "", 7, m.stem)) return false;
   for (int i = 0; i < 4; ++i) {
     const std::string p = "residual_blocks." + std::to_string(i);
     if (!make_conv(t, blob, p + ".conv1", p + ".bn1", 32, 32, 3, 1, m.conv["rb" + std::to_string(i) + "a"])) return false;
@@ -326,18 +328,14 @@ static bool build_sr(const Table& t, Blob& blob, Model& m) {
   m.conv["head"] = blob.push_gemm(gh);
   m.fin.bias[0] = BR[0];
   m.fin_heads = 1;
-  {
-    std::vector<uint16_t> pk;
-    pack_final_umma(m.fin, 1, pk);
-    std::vector<float> raw((pk.size() + 1) / 2);
-    std::memcpy(raw.data(), pk.data(), pk.size() * 2);
-    m.fin_umma_off = blob.push(raw);
-  }
+  std::vector<uint16_t> pk;
+  pack_final_umma(m.fin, 1, pk);
+  m.fin_umma_off = blob.push_half(pk);
   return true;
 }
 
 static bool build_stereo(const Table& t, Blob& blob, Model& m) {
-  if (!stem_pack(t, blob, "encoder.0.0", "encoder.0.1", 7, m.stem)) return false;
+  if (!stem_pack(t, "encoder.0.0", "encoder.0.1", 7, m.stem)) return false;
   const int dims[4][2] = {{32, 64}, {64, 128}, {128, 128}, {128, 128}};
   for (int i = 0; i < 4; ++i) {
     const std::string p = "encoder." + std::to_string(i + 1);
@@ -365,13 +363,9 @@ static bool build_stereo(const Table& t, Blob& blob, Model& m) {
     g.bias[op] = (bih[o] + bhh[o]) * sc;
   }
   m.conv["xproj"] = blob.push_gemm(g);
-  {
-    std::vector<uint16_t> pk;
-    pack_lstm_proj(g.G.data(), pk);
-    std::vector<float> raw((pk.size() + 1) / 2);
-    std::memcpy(raw.data(), pk.data(), pk.size() * 2);
-    m.wih_umma_off = blob.push(raw);
-  }
+  std::vector<uint16_t> pk;
+  pack_lstm_proj(g.G.data(), pk);
+  m.wih_umma_off = blob.push_half(pk);
   {
     std::vector<float> whh_s(256 * 64);
     for (int o = 0; o < 256; ++o)
@@ -397,13 +391,8 @@ static bool build_stereo(const Table& t, Blob& blob, Model& m) {
     m.fin.bias[s] = BF[0];
   }
   m.fin_heads = 2;
-  {
-    std::vector<uint16_t> pk;
-    pack_final_umma(m.fin, 2, pk);
-    std::vector<float> raw((pk.size() + 1) / 2);
-    std::memcpy(raw.data(), pk.data(), pk.size() * 2);
-    m.fin_umma_off = blob.push(raw);
-  }
+  pack_final_umma(m.fin, 2, pk);
+  m.fin_umma_off = blob.push_half(pk);
   return true;
 }
 
@@ -421,7 +410,7 @@ int model_create(int kind, const ar_tensor_t* tensors, int n, int device, Model*
   m->kind = kind;
   m->device = device;
   m->engine = g_engine.load();
-  m->fuse = m->engine == AR_ENGINE_UMMA ? g_fuse.load() : 0;
+  m->fuse = m->engine == AR_ENGINE_UMMA && g_fuse.load();
   Blob blob;
   bool ok = false;
   if (kind == AR_MODEL_DENOISER) ok = build_denoiser(t, blob, *m);
@@ -577,16 +566,13 @@ static int audit_act(Ctx& c, const std::string& name, const Act& a, int coff8, i
   return launch_audit(a, c.B, coff8, nch8, T, tblock, m->audit_dev + slot, c.stream);
 }
 
-static int run_conv(Ctx& c, const std::string& name, const Act& in, const Act& out, const ConvOpt& o = ConvOpt()) {
-  if (c.ar.dry) return AR_OK;
-  auto it = c.m->conv.find(name);
-  AR_CHECK(it != c.m->conv.end(), AR_ERR_INVALID, "internal: unknown conv layer " + name);
-  const ConvLayer& L = it->second;
+// Launch parameters of layer `L` (offsets into the weight blob `blob`) from `in` to `out`; `stride` = output rows per tile.
+static ConvParams conv_params(const ConvLayer& L, const float* blob, const Act& in, const Act& out, const ConvOpt& o, int B, int stride) {
   ConvParams p;
   std::memset(&p, 0, sizeof(p));
   p.in = in.h(); p.in_bs = in.bs; p.in_Tp = in.Tp; p.in_coff8 = o.in_coff8;
   p.Tin = in.T; p.Cin = L.Cin; p.taps = L.taps; p.dil = L.dil; p.pad_left = L.pad_left;
-  p.w = reinterpret_cast<const __half*>(c.m->blob + L.w_off); p.bias = c.m->blob + L.b_off; p.N = L.N; p.n_slices = L.n_slices; p.cta2 = L.cta2;
+  p.w = reinterpret_cast<const __half*>(blob + L.w_off); p.bias = blob + L.b_off; p.N = L.N; p.n_slices = L.n_slices; p.cta2 = L.cta2;
   p.mode = o.mode;
   p.out = out.h(); p.out_bs = out.bs; p.out_Tp = out.Tp; p.out_coff8 = o.out_coff8;
   p.Tout = o.Tout >= 0 ? o.Tout : out.T;
@@ -594,8 +580,17 @@ static int run_conv(Ctx& c, const std::string& name, const Act& in, const Act& o
   if (o.res) { p.res = o.res->h(); p.res_bs = o.res->bs; p.res_Tp = o.res->Tp; p.res_coff8 = 0; }
   p.lrelu = o.lrelu;
   p.out_tblock = o.out_tblock;
-  p.B = c.B;
-  p.tiles_per_item = (in.T + TILE_M - 1) / TILE_M;
+  p.B = B;
+  p.tiles_per_item = (in.T + stride - 1) / stride;
+  return p;
+}
+
+static int run_conv(Ctx& c, const std::string& name, const Act& in, const Act& out, const ConvOpt& o = ConvOpt()) {
+  if (c.ar.dry) return AR_OK;
+  auto it = c.m->conv.find(name);
+  AR_CHECK(it != c.m->conv.end(), AR_ERR_INVALID, "internal: unknown conv layer " + name);
+  const ConvLayer& L = it->second;
+  const ConvParams p = conv_params(L, c.m->blob, in, out, o, c.B, TILE_M);
   {
     ProfScope ps(CAT_CONV, c.stream, 2.0 * L.macs_per_row * (double)c.B * (double)in.T);
     AR_TRY(c.m->engine == AR_ENGINE_SIMT ? launch_conv_simt(p, c.stream) : launch_conv_umma2(p, c.stream));
@@ -612,7 +607,7 @@ static int run_conv(Ctx& c, const std::string& name, const Act& in, const Act& o
 // `_dilated_block`, stereo_separator.py:49-64, and the LSTM input projection behind the last one) or one k3 follow-up (the
 // U-Net double conv, denoiser.py:51-60, and the super-resolution residual block, super_resolution.py:104-122).  `o`
 // describes the LAST stage's output (lrelu, layout, pool copy, residual operand); intermediate stages apply LeakyReLU.
-static bool can_chain(const Ctx& c, std::initializer_list<const char*> names, bool residual = false) {
+static bool can_chain(const Ctx& c, std::initializer_list<const char*> names) {
   if (!c.m->fuse || c.m->audit || c.m->engine != AR_ENGINE_UMMA) return false;   // the audit looks at every intermediate
   bool first = true;
   int prevN = 0, Cin = 0, taps = 0, dil = 0, taps2 = 1, N[3] = {0, 0, 0}, ng = 0;
@@ -637,7 +632,6 @@ static bool can_chain(const Ctx& c, std::initializer_list<const char*> names, bo
   // 2.86, 64 -> 32 -> 32 2.14 vs 2.77; the super-resolution block 32 -> 32 -> 32 + skip ~1.9 vs 2.7 once its residual rows are
   // requested for a whole tile group ahead of the accumulator wait: model 17.5 vs 20.5 ms).  Without tile groups the narrow ones
   // lost (2.4 - 3.8 ms): profiles/README_r02.md.
-  (void)residual;
   return true;
 }
 
@@ -645,38 +639,27 @@ static int run_chain(Ctx& c, std::initializer_list<const char*> names, const Act
   if (c.ar.dry) return AR_OK;
   ChainParams cp;
   std::memset(&cp, 0, sizeof(cp));
-  cp.taps2 = 1;
+  const ConvLayer* L[3];
   double macs = 0.0;
   int g = 0;
   for (const char* n : names) {
-    const ConvLayer& L = c.m->conv.find(n)->second;
-    if (g == 0) {
-      ConvParams& p = cp.p;
-      p.in = in.h(); p.in_bs = in.bs; p.in_Tp = in.Tp; p.in_coff8 = o.in_coff8;
-      p.Tin = in.T; p.Cin = L.Cin; p.taps = L.taps; p.dil = L.dil; p.pad_left = L.pad_left;
-      p.N = L.N; p.n_slices = L.n_slices; p.cta2 = 1; p.mode = MODE_SAME; p.lrelu = 1;
-      p.B = c.B;
-    }
-    if (g == 1) cp.taps2 = L.taps;
-    cp.w[g] = reinterpret_cast<const __half*>(c.m->blob + L.w_off);
-    cp.bias[g] = c.m->blob + L.b_off;
-    cp.N[g] = L.N;
+    L[g] = &c.m->conv.at(n);
+    cp.w[g] = reinterpret_cast<const __half*>(c.m->blob + L[g]->w_off);
+    cp.bias[g] = c.m->blob + L[g]->b_off;
+    cp.N[g] = L[g]->N;
     cp.lrelu[g] = 1;
-    macs += L.macs_per_row;
+    macs += L[g]->macs_per_row;
     ++g;
   }
   cp.n_gemms = g;
+  cp.taps2 = L[1]->taps;
   cp.lrelu[g - 1] = o.lrelu;
   const int stride = chain_tile_stride(cp.taps2);
-  cp.p.tiles_per_item = (in.T + stride - 1) / stride;
-  cp.p.w = cp.w[0]; cp.p.bias = cp.bias[0];
-  cp.pl = cp.p;
-  cp.pl.N = cp.N[g - 1]; cp.pl.bias = cp.bias[g - 1]; cp.pl.lrelu = o.lrelu;
-  cp.pl.out = out.h(); cp.pl.out_bs = out.bs; cp.pl.out_Tp = out.Tp; cp.pl.out_coff8 = o.out_coff8;
-  cp.pl.Tout = o.Tout >= 0 ? o.Tout : out.T;
-  cp.pl.out_tblock = o.out_tblock;
-  if (o.pool) { cp.pl.pool = o.pool->h(); cp.pl.pool_bs = o.pool->bs; cp.pl.pool_Tp = o.pool->Tp; cp.pl.pool_coff8 = 0; }
-  if (o.res) { cp.pl.res = o.res->h(); cp.pl.res_bs = o.res->bs; cp.pl.res_Tp = o.res->Tp; cp.pl.res_coff8 = 0; }
+  // the first stage is a plain conv with LeakyReLU (launch_conv_chain takes no other); `o` describes the last stage's output
+  ConvOpt first;
+  first.in_coff8 = o.in_coff8;
+  cp.p = conv_params(*L[0], c.m->blob, in, out, first, c.B, stride);
+  cp.pl = conv_params(*L[g - 1], c.m->blob, in, out, o, c.B, stride);
   cp.head_y = o.head_y;
   cp.head_xlr = o.head_xlr;
   long long* const trace = g_chain_trace.load();
@@ -685,20 +668,31 @@ static int run_chain(Ctx& c, std::initializer_list<const char*> names, const Act
   return launch_conv_chain(cp, c.stream);
 }
 
-// A double conv (first -> second) through the fused k3 -> k3 chain when it fits, else as two launches through `mid`.
-static int run_pair(Ctx& c, const char* first, const char* second, const Act& in, int mid_channels, const Act& out, const ConvOpt& o = ConvOpt()) {
-  if (can_chain(c, {first, second}, o.res != nullptr)) {
-    ConvOpt oc = o;
-    return run_chain(c, {first, second}, in, out, oc);
+// Layers `names` in sequence from `cur` into `out`, `o` describing the last one's output and `o.in_coff8` the first one's
+// input: one fused launch when the chain kernel takes them, else one launch per layer through intermediates as wide as each
+// layer's N.  Without `out` the sequence consumes `cur` and leaves its output (as wide as the last layer) there: each tensor
+// is then allocated when its layer runs and `cur` released once read, so layer by layer at most two are alive at a time.
+static int run_seq(Ctx& c, std::initializer_list<const char*> names, Act& cur, const Act* out = nullptr, const ConvOpt& o = ConvOpt()) {
+  const bool consume = out == nullptr;
+  auto dst = [&](const char* n, bool last) { return last && !consume ? *out : c.ar.act(c.B, c.m->conv.at(n).N, cur.T); };
+  if (can_chain(c, names)) {
+    const Act y = dst(*(names.end() - 1), true);
+    AR_TRY(run_chain(c, names, cur, y, o));
+    if (consume) { c.ar.release(cur); cur = y; }
+    return AR_OK;
   }
-  Act mid = c.ar.act(c.B, mid_channels, in.T);
-  ConvOpt o1;
-  o1.in_coff8 = o.in_coff8;
-  AR_TRY(run_conv(c, first, in, mid, o1));
-  ConvOpt o2 = o;
-  o2.in_coff8 = 0;
-  AR_TRY(run_conv(c, second, mid, out, o2));
-  c.ar.release(mid);
+  Act x = cur;
+  size_t k = 0;
+  for (const char* n : names) {
+    const bool first = k == 0, last = ++k == names.size();
+    ConvOpt ok = last ? o : ConvOpt();
+    ok.in_coff8 = first ? o.in_coff8 : 0;
+    const Act y = dst(n, last);
+    AR_TRY(run_conv(c, n, x, y, ok));
+    if (!first || consume) c.ar.release(x);
+    x = y;
+  }
+  if (consume) cur = x;
   return AR_OK;
 }
 
@@ -724,33 +718,33 @@ static int denoiser_forward(Ctx& c, const float* x, float* y, int T) {
   // intermediate stays in shared memory (the bottleneck's 256-channel intermediate does not fit: two launches)
   Act cat1 = A.act(B, 128, T1), p1 = A.act(B, 64, T2);
   o = ConvOpt(); o.pool = &p1;
-  AR_TRY(run_pair(c, "enc1a", "enc1b", p0, 64, cat1, o));
+  AR_TRY(run_seq(c, {"enc1a", "enc1b"}, p0, &cat1, o));
   A.release(p0);
   Act cat2 = A.act(B, 256, T2), p2 = A.act(B, 128, T3);
   o = ConvOpt(); o.pool = &p2;
-  AR_TRY(run_pair(c, "enc2a", "enc2b", p1, 128, cat2, o));
+  AR_TRY(run_seq(c, {"enc2a", "enc2b"}, p1, &cat2, o));
   A.release(p1);
   Act b1 = A.act(B, 256, T3);
-  AR_TRY(run_pair(c, "bot_a", "bot_b", p2, 256, b1));
+  AR_TRY(run_seq(c, {"bot_a", "bot_b"}, p2, &b1));
   A.release(p2);
   // decoder level 0: up-conv writes the upper channel half of the concat buffer (skip first, :124)
   o = ConvOpt(); o.mode = MODE_INTERLEAVE2; o.lrelu = 0; o.out_coff8 = 128 / 8; o.Tout = T2;
   AR_TRY(run_conv(c, "up0", b1, cat2, o));
   A.release(b1);
   Act d0b = A.act(B, 128, T2);
-  AR_TRY(run_pair(c, "dec0a", "dec0b", cat2, 128, d0b));
+  AR_TRY(run_seq(c, {"dec0a", "dec0b"}, cat2, &d0b));
   A.release(cat2);
   o = ConvOpt(); o.mode = MODE_INTERLEAVE2; o.lrelu = 0; o.out_coff8 = 64 / 8; o.Tout = T1;
   AR_TRY(run_conv(c, "up1", d0b, cat1, o));
   A.release(d0b);
   Act d1b = A.act(B, 64, T1);
-  AR_TRY(run_pair(c, "dec1a", "dec1b", cat1, 64, d1b));
+  AR_TRY(run_seq(c, {"dec1a", "dec1b"}, cat1, &d1b));
   A.release(cat1);
   o = ConvOpt(); o.mode = MODE_INTERLEAVE2; o.lrelu = 0; o.out_coff8 = 32 / 8; o.Tout = T;
   AR_TRY(run_conv(c, "up2", d1b, cat0, o));
   A.release(d1b);
   Act f = A.act(B, 32, T);
-  AR_TRY(run_pair(c, "dec2a", "dec2b", cat0, 32, f));
+  AR_TRY(run_seq(c, {"dec2a", "dec2b"}, cat0, &f));
   A.release(cat0);
   // the cross-check engine keeps the whole transient detector on CUDA cores
   if (c.m->engine == AR_ENGINE_UMMA) {
@@ -789,7 +783,7 @@ static int sr_forward(Ctx& c, const float* x, float* y, int T) {
     // skip operand is the block's own input
     Act r2 = A.act(B, 32, T);
     ConvOpt o; o.lrelu = 0; o.res = &r;
-    AR_TRY(run_pair(c, RA[i], RB[i], r, 32, r2, o));
+    AR_TRY(run_seq(c, {RA[i], RB[i]}, r, &r2, o));
     if (i > 0) A.release(r);
     r = r2;
   }
@@ -850,50 +844,25 @@ static int stereo_encode(Ctx& c, const float* x, int T, Act& xp, bool fused_proj
     AR_TRY(launch_stem(x, B, T, m.stem, cur, 1, c.stream));
   }
   AR_TRY(audit_act(c, "stem", cur, 0, 4, T));
-  const int widths[4] = {64, 128, 128, 128};
-  static const char* const NA[4] = {"enc1a", "enc2a", "enc3a", "enc4a"};
-  static const char* const NB[4] = {"enc1b", "enc2b", "enc3b", "enc4b"};
+  // blocks 1-3 consume their input: beside a sub-batched chain's xp the encoder is the workspace peak
+  AR_TRY(run_seq(c, {"enc1a", "enc1b"}, cur));
+  AR_TRY(run_seq(c, {"enc2a", "enc2b"}, cur));
+  AR_TRY(run_seq(c, {"enc3a", "enc3b"}, cur));
   ConvOpt oxp; oxp.lrelu = 0; oxp.out_tblock = 1;   // gate pre-activations, time-blocked: the recurrence streams 4 KB runs
-  bool xp_done = false;
-  for (int i = 0; i < 4; ++i) {
-    if (i == 3 && fused_proj) {
-      if (own_xp) xp = A.act(B, 128, T);
-      if (can_chain(c, {NA[i], NB[i]})) {
-        AR_TRY(run_chain(c, {NA[i], NB[i]}, cur, xp));
-      } else {
-        Act t = A.act(B, 128, T);
-        AR_TRY(run_conv(c, NA[i], cur, t));
-        AR_TRY(run_conv(c, NB[i], t, xp));
-        A.release(t);
-      }
-      A.release(cur);
-      return AR_OK;
-    } else if (i == 3 && can_chain(c, {NA[i], NB[i], "xproj"})) {
-      // last dilated block + LSTM input projection: 128 -k3 d8-> 128 -k1-> 128 -k1-> 256 in one launch
-      if (own_xp) xp = A.act(B, 256, T);
-      AR_TRY(run_chain(c, {NA[i], NB[i], "xproj"}, cur, xp, oxp));
-      A.release(cur);
-      xp_done = true;
-    } else if (can_chain(c, {NA[i], NB[i]})) {
-      Act b = A.act(B, widths[i], T);
-      AR_TRY(run_chain(c, {NA[i], NB[i]}, cur, b));
-      A.release(cur);
-      cur = b;
-    } else {
-      Act a = A.act(B, widths[i], T);
-      AR_TRY(run_conv(c, NA[i], cur, a));
-      A.release(cur);
-      Act b = A.act(B, widths[i], T);
-      AR_TRY(run_conv(c, NB[i], a, b));
-      A.release(a);
-      cur = b;
-    }
-  }
-  if (!xp_done) {
+  if (fused_proj) {
+    if (own_xp) xp = A.act(B, 128, T);
+    AR_TRY(run_seq(c, {"enc4a", "enc4b"}, cur, &xp));
+  } else if (can_chain(c, {"enc4a", "enc4b", "xproj"})) {
+    // last dilated block + LSTM input projection: 128 -k3 d8-> 128 -k1-> 128 -k1-> 256 in one launch
+    if (own_xp) xp = A.act(B, 256, T);
+    AR_TRY(run_chain(c, {"enc4a", "enc4b", "xproj"}, cur, xp, oxp));
+  } else {
+    // the projection is not part of the sequence: xp would be alive beside both 128-channel intermediates
+    AR_TRY(run_seq(c, {"enc4a", "enc4b"}, cur));
     if (own_xp) xp = A.act(B, 256, T);   // fp16 storage costs < 0.1 dB, halves the LSTM's HBM stream
     AR_TRY(run_conv(c, "xproj", cur, xp, oxp));
-    A.release(cur);
   }
+  A.release(cur);
   return AR_OK;
 }
 
@@ -941,9 +910,9 @@ static int stereo_decode(Ctx& c, const Act& h, float* y, int T, bool h_owned) {
   // (the 64-channel intermediate stays in shared memory), else two launches through a 64-channel tensor
   Act d2 = A.act(B, 64, T);
   ConvOpt o;
-  AR_TRY(run_pair(c, "dec1L", "dec2L", d0, 64, d2, o));
+  AR_TRY(run_seq(c, {"dec1L", "dec2L"}, d0, &d2, o));
   o.in_coff8 = 128 / 8; o.out_coff8 = 32 / 8;
-  AR_TRY(run_pair(c, "dec1R", "dec2R", d0, 64, d2, o));
+  AR_TRY(run_seq(c, {"dec1R", "dec2R"}, d0, &d2, o));
   A.release(d0);
   if (!A.dry) {
     const int coff[2] = {0, 32 / 8};
@@ -1183,12 +1152,9 @@ int debug_conv(const float* x, const float* w_host, const float* bias_host, floa
   Act in = A.act(B, Cin, T), out = A.act(B, Cout, T);
   int rc = launch_plain_to_c4(x, B, Cin, T, in, stream);
   if (rc == AR_OK) {
-    ConvParams p;
-    std::memset(&p, 0, sizeof(p));
-      p.in = in.h(); p.in_bs = in.bs; p.in_Tp = in.Tp; p.Tin = T; p.Cin = Cin; p.taps = L.taps; p.dil = L.dil; p.pad_left = g.pad_left;
-    p.w = reinterpret_cast<const __half*>(dblob + L.w_off); p.bias = dblob + L.b_off; p.N = L.N; p.n_slices = L.n_slices; p.cta2 = L.cta2; p.mode = MODE_SAME;
-    p.out = out.h(); p.out_bs = out.bs; p.out_Tp = out.Tp; p.Tout = T; p.lrelu = lrelu;
-    p.B = B; p.tiles_per_item = (T + TILE_M - 1) / TILE_M;
+    ConvOpt o;
+    o.lrelu = lrelu;
+    const ConvParams p = conv_params(L, dblob, in, out, o, B, TILE_M);
     rc = engine == AR_ENGINE_SIMT ? launch_conv_simt(p, stream) : launch_conv_umma2(p, stream);
   }
   if (rc == AR_OK) rc = launch_c4_to_plain(out, B, Cout, T, y, stream);

@@ -12,7 +12,7 @@ MIN_SNR_DB = 60.0   # ... or >= 60 dB SNR; the tests demand both unless stated
 
 
 def make_model(name, sd, engine=_lib.ENGINE_UMMA, device="cuda", fusion=1):
-    """fusion: 0 layer by layer, 1 / True the product default, 2 every fused chain that fits (ar_set_fusion)."""
+    """fusion: 0 / False layer by layer, 1 / True every fused chain that fits, the product default (ar_set_fusion)."""
     m = CLS[name]()
     m.load_state_dict(sd, strict=True)
     m = m.to(device).eval()

@@ -131,9 +131,10 @@ def test_fused_chains_match_layer_by_layer(weight_sets, B, T, weights):
 @pytest.mark.parametrize("weights", ["benign", "calibrated"])
 @pytest.mark.parametrize("name", ["denoiser", "super_resolution"])
 @pytest.mark.parametrize("B,T", [(1, 8), (2, 125), (1, 126), (3, 127), (1, 252), (2, 253), (1, 1009), (5, 4099), (150, 1100)])
-def test_fused_double_convs_match_layer_by_layer(weight_sets, name, B, T, weights):
-    """The fused k3 -> k3 launches (U-Net double convs with the max-pool copy, super-resolution residual blocks with the
-    skip add; conv_chain.cu, tile stride 126) compute the same fp16-rounded intermediates as the layer-by-layer launches.
+def test_fused_double_convs_match_fusion_off(weight_sets, name, B, T, weights):
+    """With fusion on (the product default), the fused k3 -> k3 launches (U-Net double convs with the max-pool copy,
+    super-resolution residual blocks with the skip add; conv_chain.cu, tile stride 126) compute the same fp16-rounded
+    intermediates as the layer-by-layer launches of fusion off.
     Lengths around the 126-row tile stride and its multiples (at every U-Net level: T, T/2, T/4), odd tile counts (idle peer
     CTA), and B=150 for the steady-state pipeline.  The denoiser is bitwise equal.  The super-resolution output head is
     the one fused path that legitimately differs: fused behind hf_emphasis it runs on the tensor core, layer by layer on
@@ -141,7 +142,7 @@ def test_fused_double_convs_match_layer_by_layer(weight_sets, name, B, T, weight
     float64 head restatement of tests/layer_ref.py on the tapped hf_emphasis output of the layer-by-layer path, on every
     item of the batch, and (benign weights) to the layer-by-layer output within 2e-5 and 90 dB."""
     sd = weight_sets[weights][name]
-    fused = make_model(name, sd, fusion=2)      # every pair that fits, not only the measured-faster ones
+    fused = make_model(name, sd, fusion=1)
     plain = make_model(name, sd, fusion=0)
     x = make_input(B, T, seed=B * 11 + T)
     with torch.no_grad():
@@ -275,10 +276,10 @@ def _forward_filled(m, x, out_shape, audit=False, window=None):
 OUT = {"denoiser": lambda B, T: (B, 1, T), "super_resolution": lambda B, T: (B, 1, 2 * T), "stereo": lambda B, T: (B, 2, T)}
 
 
-@pytest.mark.parametrize("mode", ["fusion0", "fusion1", "fusion2", "audit"])
+@pytest.mark.parametrize("mode", ["fusion0", "fusion1", "audit"])
 @pytest.mark.parametrize("name", ["denoiser", "super_resolution", "stereo"])
 def test_forwards_ignore_workspace_contents(state_dicts, name, mode):
-    fusion = {"fusion0": 0, "fusion1": 1, "fusion2": 2, "audit": 1}[mode]
+    fusion = {"fusion0": 0, "fusion1": 1, "audit": 1}[mode]
     m = make_model(name, state_dicts[name], fusion=fusion)
     batches = [2] if name != "stereo" else [3, 2 * _sm_count() + 8, 8 * _sm_count() + 13]
     for B in batches:

@@ -30,6 +30,16 @@ def test_library_exports_every_declared_symbol():
     assert _lib.lib().ar_version() >= 100
 
 
+def test_fusion_is_on_or_off():
+    """ar_set_fusion takes 0 (layer by layer) or 1 (fused, the default); any other value is refused."""
+    from ml_audio_restoration_b200 import _lib
+    L = _lib.lib()
+    for bad in (-1, 2, 3):
+        assert L.ar_set_fusion(bad) == _lib.AR_ERR_INVALID
+    assert L.ar_set_fusion(0) == _lib.AR_OK
+    assert L.ar_set_fusion(1) == _lib.AR_OK
+
+
 def test_library_is_sm100a_native_code():
     """The shipped library is sm_100a machine code with the Blackwell instructions the design rests on (DESIGN.md 3): tcgen05.mma
     (UTCHMMA, 1- and 2-CTA), TMEM loads (LDTM), bulk-async TMA copies and L2 prefetches (UBLKCP / UBLKPF), the LSTM's warp MMA

@@ -17,7 +17,7 @@ def main():
     B = int(sys.argv[1]) if len(sys.argv) > 1 else 148
     T = int(sys.argv[2]) if len(sys.argv) > 2 else 44100
     which = sys.argv[3] if len(sys.argv) > 3 else "stereo"
-    fusion = int(sys.argv[4]) if len(sys.argv) > 4 else 1      # 2: also the k3 -> k3 chains that are off in the product path
+    fusion = int(sys.argv[4]) if len(sys.argv) > 4 else 1      # 0: layer by layer (nothing to trace)
     _lib.check(_lib.lib().ar_set_fusion(fusion))
     torch.manual_seed(0)
     m = {"stereo": StereoSeparator, "sr": lambda: AudioSuperResolution(upscale_factor=2), "denoiser": AudioDenoiser}[which]().cuda().eval()

@@ -1,4 +1,4 @@
-"""Two forwards of one model (target of ncu captures).   python tools/probe_forward.py stereo|sr|denoiser [B] [T] [fusion level]"""
+"""Two forwards of one model (target of ncu captures).   python tools/probe_forward.py stereo|sr|denoiser [B] [T] [fusion 0|1]"""
 import sys, os, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from oracle.weights import make_state_dict, make_input

@@ -1,5 +1,5 @@
-"""Times the denoiser / super-resolution forwards at a bench sub-batch for the fusion levels of ar_set_fusion
-(0 layer by layer, 1 product default, 2 every fused chain that fits), CUDA events, median of 5.
+"""Times the denoiser / super-resolution forwards at a bench sub-batch with ar_set_fusion off and on
+(0 layer by layer, 1 every fused chain that fits, the product default), CUDA events, median of 5.
    python tools/probe_fusion.py [B] [T]"""
 import sys, os, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -12,7 +12,7 @@ L = _lib.lib()
 for name, cls in (("denoiser", AudioDenoiser), ("super_resolution", lambda: AudioSuperResolution(upscale_factor=2)), ("stereo", StereoSeparator)):
     x = make_input(B if name != "stereo" else B // 4, T).cuda()
     outs = {}
-    for level in (0, 1, 2):
+    for level in (0, 1):
         _lib.check(L.ar_set_fusion(level))
         m = cls(); m.load_state_dict(make_state_dict(name)); m = m.cuda().eval()
         with torch.no_grad():
