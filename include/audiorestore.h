@@ -121,6 +121,27 @@ int ar_stereo_forward_window(ar_model_t m, const float* x, float* y, int B, int 
                              const float* state_in, float* state_out,
                              void* workspace, size_t workspace_bytes, void* stream);
 
+/* ar_stereo_forward_window for B windows that hand their state on at different steps (lockstep whole-file-exact mode over
+ * many files): state_pos is a HOST array of B entries, lstm_start < state_pos[b] <= T, any integers; state_out[b] receives
+ * (h, c) after step state_pos[b] - 1 while the scan of item b runs on to T in the same launch.  The array is checked on the
+ * host and uploaded into the workspace (counted by ar_model_workspace_bytes) on `stream`; no host synchronisation.
+ * Outputs and states equal those of ar_stereo_forward_window on the same batch with state_pos = state_pos[b]. */
+int ar_stereo_forward_window_multi(ar_model_t m, const float* x, float* y, int B, int T, int lstm_start, const int* state_pos,
+                                   const float* state_in, float* state_out,
+                                   void* workspace, size_t workspace_bytes, void* stream);
+
+/* Window gather / kept-range scatter (lockstep whole-file-exact mode, one launch per direction for all files):
+ *   ar_gather_windows : dst[b][0][0..W) = src[offsets[b] .. offsets[b] + W)             (0 <= offsets[b] <= src_len - W)
+ *   ar_scatter_kept   : out[dst_offsets[2b + c] + j] = y[b][c][lo[b] + j], j < len[b], c = 0, 1  (y is [B,2,W];
+ *                       0 <= lo[b], lo[b] + len[b] <= W, dst_offsets[2b + c] + len[b] <= out_len)
+ * Offsets and ranges are HOST arrays, checked on the host and uploaded into `workspace` (>= B * AR_WINDOW_IO_BYTES_PER_ITEM
+ * device bytes, not reused by the caller before the launch has run) on `stream`; no host synchronisation. */
+#define AR_WINDOW_IO_BYTES_PER_ITEM 24
+int ar_gather_windows(const float* src, int64_t src_len, const int64_t* offsets, int B, int W, float* dst,
+                      void* workspace, size_t workspace_bytes, void* stream);
+int ar_scatter_kept(const float* y, int B, int W, const int64_t* dst_offsets, const int* lo, const int* len, float* out,
+                    int64_t out_len, void* workspace, size_t workspace_bytes, void* stream);
+
 /* denoise -> (super-res) -> stereo on a batch of equal-length chunks
  * (the three model applications of inference.py:59-61,73-75,93-95).  sr may be NULL
  * (enable_super_resolution=False): y is [B,2,T] instead of [B,2,2T].

@@ -18,6 +18,7 @@ AR_OK, AR_ERR_INVALID, AR_ERR_WEIGHTS, AR_ERR_CUDA, AR_ERR_WORKSPACE = 0, 1, 2, 
 MODEL_DENOISER, MODEL_SUPER_RES, MODEL_STEREO = 0, 1, 2
 ENGINE_UMMA, ENGINE_SIMT = 0, 1
 NORMALIZE_SCRATCH_BYTES = 16384
+WINDOW_IO_BYTES_PER_ITEM = 24
 AUDIT_MAX_LAYERS = 64
 HALF_MAX = 65504.0
 PROFILE_CATEGORIES = ("conv", "lstm", "stem", "tail", "normalize", "chunk")
@@ -45,6 +46,12 @@ _SIGNATURES = {
                                           C.c_void_p, C.c_size_t, C.c_void_p]),
     "ar_stereo_forward_window": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p,
                                            C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "ar_stereo_forward_window_multi": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                                 C.POINTER(C.c_int), C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "ar_gather_windows": (C.c_int, [C.c_void_p, C.c_int64, C.POINTER(C.c_int64), C.c_int, C.c_int, C.c_void_p, C.c_void_p,
+                                    C.c_size_t, C.c_void_p]),
+    "ar_scatter_kept": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_int64), C.POINTER(C.c_int), C.POINTER(C.c_int),
+                                  C.c_void_p, C.c_int64, C.c_void_p, C.c_size_t, C.c_void_p]),
     "ar_chain_create": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_void_p)]),
     "ar_chain_destroy": (None, [C.c_void_p]),
     "ar_chain_workspace_bytes": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_size_t)]),

@@ -37,7 +37,8 @@ int launch_filtfilt(const float* x, float scale, const float* add1, const float*
 int model_create(int kind, const ar_tensor_t* tensors, int n, int device, Model** out);
 int model_workspace_bytes(const Model* m, int B, int T, size_t* bytes);
 int model_forward(const Model* m, const float* x, float* y, int B, int T, const float* st_in, float* st_out, void* ws,
-                  size_t ws_bytes, cudaStream_t stream, int lstm_start = 0, int state_pos = -1);
+                  size_t ws_bytes, cudaStream_t stream, int lstm_start = 0, int state_pos = -1,
+                  const int* state_pos_host = nullptr);
 int chain_workspace_bytes(const Model* den, const Model* sr, const Model* st, int B, int T, size_t* bytes);
 int chain_forward(const Model* den, const Model* sr, const Model* st, const float* x, float* y, int B, int T, void* ws,
                   size_t ws_bytes, cudaStream_t stream);
@@ -164,6 +165,16 @@ int ar_stereo_forward_window(ar_model_t m, const float* x, float* y, int B, int 
                            reinterpret_cast<cudaStream_t>(stream), lstm_start, state_pos);
 }
 
+int ar_stereo_forward_window_multi(ar_model_t m, const float* x, float* y, int B, int T, int lstm_start, const int* state_pos,
+                                   const float* state_in, float* state_out, void* workspace, size_t workspace_bytes,
+                                   void* stream) {
+  AR_CHECK(m && ar::model_kind(reinterpret_cast<ar::Model*>(m)) == AR_MODEL_STEREO, AR_ERR_INVALID,
+           "ar_stereo_forward_window_multi: not a stereo model");
+  AR_CHECK(state_pos != nullptr, AR_ERR_INVALID, "ar_stereo_forward_window_multi: null state_pos");
+  return ar::model_forward(reinterpret_cast<ar::Model*>(m), x, y, B, T, state_in, state_out, workspace, workspace_bytes,
+                           reinterpret_cast<cudaStream_t>(stream), lstm_start, -1, state_pos);
+}
+
 int ar_chain_create(ar_model_t denoiser, ar_model_t sr, ar_model_t stereo, ar_chain_t* out) {
   AR_CHECK(out && denoiser && stereo, AR_ERR_INVALID, "ar_chain_create: denoiser and stereo models are required");
   AR_CHECK(ar_model_kind(denoiser) == AR_MODEL_DENOISER && ar_model_kind(stereo) == AR_MODEL_STEREO &&
@@ -220,6 +231,20 @@ int ar_overlap_add(const float* y, float* out, int64_t n, int n_chunks, int chan
   AR_CHECK(y && out && n_chunks == total && channels >= 1 && rate >= 1, AR_ERR_INVALID, "ar_overlap_add: bad argument");
   ar::ProfScope ps(ar::CAT_CHUNK, reinterpret_cast<cudaStream_t>(stream), 0.0);
   return ar::launch_ola(y, out, n, n_chunks, channels, chunk_size, overlap, rate, reinterpret_cast<cudaStream_t>(stream));
+}
+
+int ar_gather_windows(const float* src, int64_t src_len, const int64_t* offsets, int B, int W, float* dst, void* workspace,
+                      size_t workspace_bytes, void* stream) {
+  ar::ProfScope ps(ar::CAT_CHUNK, reinterpret_cast<cudaStream_t>(stream), 0.0);
+  return ar::launch_gather_windows(src, src_len, reinterpret_cast<const long long*>(offsets), B, W, dst, workspace, workspace_bytes,
+                                   reinterpret_cast<cudaStream_t>(stream));
+}
+
+int ar_scatter_kept(const float* y, int B, int W, const int64_t* dst_offsets, const int* lo, const int* len, float* out,
+                    int64_t out_len, void* workspace, size_t workspace_bytes, void* stream) {
+  ar::ProfScope ps(ar::CAT_CHUNK, reinterpret_cast<cudaStream_t>(stream), 0.0);
+  return ar::launch_scatter_kept(y, B, W, reinterpret_cast<const long long*>(dst_offsets), lo, len, out, out_len, workspace,
+                                 workspace_bytes, reinterpret_cast<cudaStream_t>(stream));
 }
 
 int ar_profile_enable(int on) { return ar::prof_enable(on); }

@@ -36,11 +36,14 @@ __device__ __forceinline__ long long tb_off(int t) {
   return (long long)(tr >> 3) * (32 * 64) + (tr & 7) * 8;
 }
 
-template <int S, int PF>
+// CAP: sequence b hands (h, c) to state_out[b] after local step cap[b] - 1 (cap[b] >= T: after the last step) and its
+// scan continues.  A compile-time variant: the compare costs a share of the ~77-instruction step, so the scans without a
+// per-sequence capture position keep the code they had.
+template <int S, int PF, bool CAP = false>
 __global__ void __launch_bounds__(256, (S <= 2) ? 2 : 1)
 lstm_kernel(const __half* __restrict__ xp, long long xp_bs, int xp_Tp, const float* __restrict__ whh,
             __half* __restrict__ hout, long long h_bs, int h_Tp, int B, int T,
-            const float* __restrict__ state_in, float* __restrict__ state_out) {
+            const float* __restrict__ state_in, float* __restrict__ state_out, const int* __restrict__ cap = nullptr) {
   __shared__ __align__(16) float hbuf[2][S][LSTM_H];
   __shared__ __align__(16) float hstage[2][S][LSTM_BLK][LSTM_H];
   const int tid = threadIdx.x;
@@ -60,9 +63,11 @@ lstm_kernel(const __half* __restrict__ xp, long long xp_bs, int xp_Tp, const flo
 
   float c[S];
   const __half* xrow[S];
+  int capt[S];
 #pragma unroll
   for (int s = 0; s < S; ++s) {
     const int b = min(seq0 + s, B - 1);  // surplus slots replay the last sequence, stores are masked
+    if constexpr (CAP) capt[s] = seq0 + s < B ? min(cap[b], T) : 0;
     c[s] = 0.f;
     float h0 = 0.f;
     if (state_in != nullptr) {
@@ -135,6 +140,12 @@ lstm_kernel(const __half* __restrict__ xp, long long xp_bs, int xp_Tp, const flo
             hlast[s] = h;
             hbuf[cur ^ 1][s][unit] = h;
             hstage[sb][s][t & 7][unit] = h;
+            if constexpr (CAP) {
+              if (t == capt[s] - 1) {
+                state_out[(long long)(seq0 + s) * 2 * LSTM_H + unit] = h;
+                state_out[(long long)(seq0 + s) * 2 * LSTM_H + LSTM_H + unit] = c[s];
+              }
+            }
           }
         }
         __syncthreads();
@@ -164,7 +175,7 @@ lstm_kernel(const __half* __restrict__ xp, long long xp_bs, int xp_Tp, const flo
     run_block(xa, xb, t0);
     if (t0 + PF < T) run_block(xb, xa, t0 + PF);
   }
-  if (state_out != nullptr && gate == 0) {
+  if (!CAP && state_out != nullptr && gate == 0) {
 #pragma unroll
     for (int s = 0; s < S; ++s) {
       const int b = seq0 + s;
@@ -216,11 +227,11 @@ struct LwGeom {
   static constexpr int SMEM = 2 * XBUF * 2 + 2 * LSTM_BLK * HSTEP * 4 + 2 * NSEQ * LM_HS * 2;
 };
 
-template <int NSEQ>
+template <int NSEQ, bool CAP = false>
 __global__ void __launch_bounds__(LW_THREADS, 2)
 lstm_mmaw_kernel(const __half* __restrict__ xp, long long xp_bs, int xp_Tp, const float* __restrict__ whh,
                  __half* __restrict__ hout, long long h_bs, int h_Tp, int B, int T,
-                 const float* __restrict__ state_in, float* __restrict__ state_out) {
+                 const float* __restrict__ state_in, float* __restrict__ state_out, const int* __restrict__ cap = nullptr) {
   static_assert(NSEQ == 4 || NSEQ == 8, "four (duplicated columns) or eight sequences per CTA");
   using G = LwGeom<NSEQ>;
   constexpr int CELLS = NSEQ / 4;                              // cells per recurrence thread
@@ -289,10 +300,12 @@ lstm_mmaw_kernel(const __half* __restrict__ xp, long long xp_bs, int xp_Tp, cons
   const int upos = h_exchange_pos(unit);
   // this thread's cells: (unit, sequence tig * CELLS + j); the sequence of cell j sits in accumulator column 2 tig + j
   float c[CELLS], hl[CELLS];
+  int capt[CELLS];
 #pragma unroll
   for (int j = 0; j < CELLS; ++j) {
     const int seq = tig * CELLS + j;
     const int bq = min(seq0 + seq, B - 1);
+    if constexpr (CAP) capt[j] = seq0 + seq < B ? min(cap[bq], T) : 0;
     c[j] = 0.f;
     hl[j] = 0.f;
     if (state_in != nullptr) {
@@ -343,12 +356,22 @@ lstm_mmaw_kernel(const __half* __restrict__ xp, long long xp_bs, int xp_Tp, cons
       hst[k * G::HSTEP + hoff + j * LM_HST] = hl[j];
     }
   };
+  auto capture = [&](int t) {                        // CAP: (h, c) of the cells whose capture step t is
+#pragma unroll
+    for (int j = 0; j < CELLS; ++j)
+      if (t == capt[j] - 1) {
+        const long long b = seq0 + tig * CELLS + j;
+        state_out[b * 2 * LSTM_H + unit] = hl[j];
+        state_out[b * 2 * LSTM_H + LSTM_H + unit] = c[j];
+      }
+  };
   for (int blk = 0; blk < nfull; ++blk) {
     const __half* xb = xs + (blk & 1) * G::XBUF;
     float* hst = hstage + (blk & 1) * (LSTM_BLK * G::HSTEP);
 #pragma unroll
     for (int k = 0; k < LSTM_BLK; ++k) {
       step(xb, hst, k);
+      if constexpr (CAP) capture(blk * LSTM_BLK + k);
       if (k < LSTM_BLK - 1) asm volatile("bar.sync 2, %0;" ::"n"(LW_REC) : "memory");
       else asm volatile("bar.sync 1, %0;" ::"n"(LW_THREADS) : "memory");
     }
@@ -361,12 +384,13 @@ lstm_mmaw_kernel(const __half* __restrict__ xp, long long xp_bs, int xp_Tp, cons
     for (int k = 0; k < LSTM_BLK - 1; ++k) {
       if (k < nst) {   // uniform
         step(xb, hst, k);
+        if constexpr (CAP) capture(nfull * LSTM_BLK + k);
         asm volatile("bar.sync 2, %0;" ::"n"(LW_REC) : "memory");
       }
     }
     asm volatile("bar.sync 1, %0;" ::"n"(LW_THREADS) : "memory");
   }
-  if (state_out != nullptr) {
+  if (!CAP && state_out != nullptr) {
 #pragma unroll
     for (int j = 0; j < CELLS; ++j) {
       const int b = seq0 + tig * CELLS + j;
@@ -378,33 +402,46 @@ lstm_mmaw_kernel(const __half* __restrict__ xp, long long xp_bs, int xp_Tp, cons
   }
 }
 
-template <int NSEQ>
+template <int NSEQ, bool CAP>
 static int launch_lstm_mmaw(const Act& xp, const float* whh, const Act& h_out, int B, int T, const float* state_in, float* state_out,
-                            cudaStream_t stream) {
+                            const int* cap, cudaStream_t stream) {
   static DeviceOnce attrs;
   if (attrs.pending()) {
-    AR_CUDA_OK(cudaFuncSetAttribute(lstm_mmaw_kernel<NSEQ>, cudaFuncAttributeMaxDynamicSharedMemorySize, LwGeom<NSEQ>::SMEM));
+    AR_CUDA_OK(cudaFuncSetAttribute(lstm_mmaw_kernel<NSEQ, CAP>, cudaFuncAttributeMaxDynamicSharedMemorySize, LwGeom<NSEQ>::SMEM));
     // two CTAs (53 / 103 KB each) must fit: ask for the largest shared-memory carve-out, the driver's default heuristic sizes
     // it for ONE CTA and the second recurrence of the SM would run after the first instead of under it
-    AR_CUDA_OK(cudaFuncSetAttribute(lstm_mmaw_kernel<NSEQ>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    AR_CUDA_OK(cudaFuncSetAttribute(lstm_mmaw_kernel<NSEQ, CAP>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     attrs.done();
   }
-  lstm_mmaw_kernel<NSEQ><<<(B + NSEQ - 1) / NSEQ, LW_THREADS, LwGeom<NSEQ>::SMEM, stream>>>(xp.h(), xp.bs, xp.Tp, whh, h_out.h(), h_out.bs,
-                                                                                      h_out.Tp, B, T, state_in, state_out);
+  lstm_mmaw_kernel<NSEQ, CAP><<<(B + NSEQ - 1) / NSEQ, LW_THREADS, LwGeom<NSEQ>::SMEM, stream>>>(
+      xp.h(), xp.bs, xp.Tp, whh, h_out.h(), h_out.bs, h_out.Tp, B, T, state_in, state_out, cap);
+  return AR_OK;
+}
+
+template <bool CAP>
+static int launch_lstm_t(const Act& xp, const float* whh, const Act& h_out, int B, int T, const float* state_in, float* state_out,
+                         const int* cap, cudaStream_t stream) {
+  // One sequence per CTA on CUDA cores (two CTAs per SM) while that covers the batch; beyond two sequences per SM the
+  // tensor-core kernel, two CTAs per SM: four sequences per CTA up to 8 per SM, eight per CTA beyond that.
+  if (B > 8 * sm_count()) {
+    AR_TRY((launch_lstm_mmaw<8, CAP>(xp, whh, h_out, B, T, state_in, state_out, cap, stream)));
+  } else if (B > 2 * sm_count()) {
+    AR_TRY((launch_lstm_mmaw<4, CAP>(xp, whh, h_out, B, T, state_in, state_out, cap, stream)));
+  } else {
+    lstm_kernel<1, 8, CAP><<<B, 256, 0, stream>>>(xp.h(), xp.bs, xp.Tp, whh, h_out.h(), h_out.bs, h_out.Tp, B, T, state_in,
+                                                  state_out, cap);
+  }
   return AR_OK;
 }
 
 int launch_lstm(const Act& xp, const float* whh, const Act& h_out, int B, int T, const float* state_in, float* state_out,
-                cudaStream_t stream) {
+                const int* cap, cudaStream_t stream) {
   AR_CHECK(T >= 1 && B >= 1, AR_ERR_INVALID, "lstm: empty input");
-  // One sequence per CTA on CUDA cores (two CTAs per SM) while that covers the batch; beyond two sequences per SM the
-  // tensor-core kernel, two CTAs per SM: four sequences per CTA up to 8 per SM, eight per CTA beyond that.
-  if (B > 8 * sm_count()) {
-    AR_TRY(launch_lstm_mmaw<8>(xp, whh, h_out, B, T, state_in, state_out, stream));
-  } else if (B > 2 * sm_count()) {
-    AR_TRY(launch_lstm_mmaw<4>(xp, whh, h_out, B, T, state_in, state_out, stream));
+  AR_CHECK(cap == nullptr || state_out != nullptr, AR_ERR_INVALID, "lstm: per-sequence capture needs state_out");
+  if (cap != nullptr) {
+    AR_TRY(launch_lstm_t<true>(xp, whh, h_out, B, T, state_in, state_out, cap, stream));
   } else {
-    lstm_kernel<1, 8><<<B, 256, 0, stream>>>(xp.h(), xp.bs, xp.Tp, whh, h_out.h(), h_out.bs, h_out.Tp, B, T, state_in, state_out);
+    AR_TRY(launch_lstm_t<false>(xp, whh, h_out, B, T, state_in, state_out, nullptr, stream));
   }
   AR_CUDA_OK(cudaGetLastError());
   return AR_OK;

@@ -77,8 +77,10 @@ struct LstmProjArgs {
   int B, T;
   const float* state_in;
   float* state_out;
+  const int* cap;         // CAP: per-sequence capture step (lstm_kernel in lstm.cu)
 };
 
+template <bool CAP>
 __global__ void __launch_bounds__(LP_THREADS, 1) lstm_proj_kernel(const __grid_constant__ LstmProjArgs a) {
   extern __shared__ __align__(1024) uint8_t smem[];
   const uint32_t sbase = smem_u32(smem);
@@ -260,9 +262,11 @@ __global__ void __launch_bounds__(LP_THREADS, 1) lstm_proj_kernel(const __grid_c
     const int upos = h_exchange_pos(unit);
     const int sl0 = g * 8 + tig * 2;               // this thread's cells: (unit, CTA-local sequences sl0, sl0 + 1)
     float c[2], hl[2];
+    int capt[2];
 #pragma unroll
     for (int j = 0; j < 2; ++j) {
       const int bq = min(seq0 + sl0 + j, B - 1);
+      if constexpr (CAP) capt[j] = seq0 + sl0 + j < B ? min(a.cap[bq], T) : 0;
       c[j] = 0.f;
       hl[j] = 0.f;
       if (a.state_in != nullptr) {
@@ -317,6 +321,15 @@ __global__ void __launch_bounds__(LP_THREADS, 1) lstm_proj_kernel(const __grid_c
         if (k < nst) {   // uniform; always true except in a ragged last block
           if ((k & 1) == 0) mbar_wait(slot_full(k >> 1), (uint32_t)blk & 1u);
           step(hst, k);
+          if constexpr (CAP) {
+#pragma unroll
+            for (int j = 0; j < 2; ++j)
+              if (blk * LSTM_BLK + k == capt[j] - 1) {
+                const long long b = seq0 + sl0 + j;
+                a.state_out[b * 2 * LSTM_H + unit] = hl[j];
+                a.state_out[b * 2 * LSTM_H + LSTM_H + unit] = c[j];
+              }
+          }
           if (g == 0) asm volatile("bar.sync 2, 256;" ::: "memory");
           else asm volatile("bar.sync 3, 256;" ::: "memory");
           if ((k & 1) && g_lead) mbar_arrive(slot_free(k >> 1));          // this group is past steps 2 q, 2 q + 1: slot q may be rewritten
@@ -324,7 +337,7 @@ __global__ void __launch_bounds__(LP_THREADS, 1) lstm_proj_kernel(const __grid_c
       }
       if (g_lead) mbar_arrive(blk_done(blk & 1));
     }
-    if (a.state_out != nullptr) {
+    if (!CAP && a.state_out != nullptr) {
 #pragma unroll
       for (int j = 0; j < 2; ++j) {
         const int b = seq0 + sl0 + j;
@@ -357,20 +370,23 @@ void pack_lstm_proj(const float* G /* [128 cin][256 n] */, std::vector<uint16_t>
 }
 
 int launch_lstm_proj(const Act& x, const __half* wih_packed, const float* bias, const float* whh, const Act& h_out, int B, int T,
-                     const float* state_in, float* state_out, cudaStream_t stream) {
+                     const float* state_in, float* state_out, const int* cap, cudaStream_t stream) {
   AR_CHECK(T >= 1 && B >= 1 && x.C == LP_K, AR_ERR_INVALID, "lstm_proj: bad input");
+  AR_CHECK(cap == nullptr || state_out != nullptr, AR_ERR_INVALID, "lstm_proj: per-sequence capture needs state_out");
   static DeviceOnce attrs;
   if (attrs.pending()) {
-    AR_CUDA_OK(cudaFuncSetAttribute(lstm_proj_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, LP_SMEM));
+    AR_CUDA_OK(cudaFuncSetAttribute(lstm_proj_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, LP_SMEM));
+    AR_CUDA_OK(cudaFuncSetAttribute(lstm_proj_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, LP_SMEM));
     attrs.done();
   }
   LstmProjArgs a;
   a.x = x.h(); a.x_bs = x.bs; a.x_Tp = x.Tp;
   a.wih = wih_packed; a.bias = bias; a.whh = whh;
   a.hout = h_out.h(); a.h_bs = h_out.bs; a.h_Tp = h_out.Tp;
-  a.B = B; a.T = T; a.state_in = state_in; a.state_out = state_out;
+  a.B = B; a.T = T; a.state_in = state_in; a.state_out = state_out; a.cap = cap;
 
-  lstm_proj_kernel<<<(B + LP_SEQ - 1) / LP_SEQ, LP_THREADS, LP_SMEM, stream>>>(a);
+  if (cap != nullptr) lstm_proj_kernel<true><<<(B + LP_SEQ - 1) / LP_SEQ, LP_THREADS, LP_SMEM, stream>>>(a);
+  else lstm_proj_kernel<false><<<(B + LP_SEQ - 1) / LP_SEQ, LP_THREADS, LP_SMEM, stream>>>(a);
   AR_CUDA_OK(cudaGetLastError());
   return AR_OK;
 }

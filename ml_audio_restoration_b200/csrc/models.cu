@@ -822,7 +822,9 @@ static int sr_forward(Ctx& c, const float* x, float* y, int T) {
 // The LSTM scan covers steps [w.lstm_start, T) (hidden states before it are zero) starting from `state_in`, and
 // `state_out` receives (h, c) after step w.state_pos - 1: the window parameters of the whole-file-exact chunked mode
 // (ar_stereo_forward_window), where a segment carries conv halos on both sides of the range whose state it hands on.
-struct LstmWindow { int lstm_start = 0, state_pos = -1; };
+// With `cap` (device, [B]) item b hands its state on after step lstm_start + cap[b] - 1 instead, in the same launch
+// (ar_stereo_forward_window_multi: windows of different files, each handing on at its own position).
+struct LstmWindow { int lstm_start = 0, state_pos = -1; const int* cap = nullptr; };
 
 // The forward in three phases, so that the chain (chain_forward below) can run them on different batch splits:
 //   encode  stem + dilated encoder + LSTM input projection  x[B,1,T] -> xp (gate pre-activations, time-blocked fp16)
@@ -874,21 +876,24 @@ static int stereo_scan(Ctx& c, const Act& xp, const Act& h, int T, const float* 
   ProfScope ps(CAT_LSTM, c.stream, 2.0 * (fused_proj ? 16384 + 32768 : 16384) * (double)B * (T - w.lstm_start), w.state_pos < T ? 2 : 1);
   // a scan over steps [t0, t1) is the same kernel on base pointers advanced by t0 rows (t0 % 8 == 0 keeps the 8-step
   // blocks of the time-blocked pre-activations aligned)
-  auto scan = [&](int t0, int t1, const float* st_in, float* st_out) {
+  auto scan = [&](int t0, int t1, const float* st_in, float* st_out, const int* cap = nullptr) {
     Act xs = xp, hs = h;
     hs.base = h.h() + (long long)t0 * 8;
     xs.T = hs.T = t1 - t0;
     if (fused_proj) {
       xs.base = xp.h() + (long long)t0 * 8;
       return launch_lstm_proj(xs, reinterpret_cast<const __half*>(m.blob + m.wih_umma_off), m.blob + m.conv.at("xproj").b_off,
-                              m.blob + m.whh_off, hs, B, t1 - t0, st_in, st_out, c.stream);
+                              m.blob + m.whh_off, hs, B, t1 - t0, st_in, st_out, cap, c.stream);
     }
     xs.base = xp.h() + (long long)(t0 / 8) * 32 * 64;
-    return launch_lstm(xs, m.blob + m.whh_off, hs, B, t1 - t0, st_in, st_out, c.stream);
+    return launch_lstm(xs, m.blob + m.whh_off, hs, B, t1 - t0, st_in, st_out, cap, c.stream);
   };
   if (w.lstm_start > 0)   // rows [0, lstm_start) of all 8 chunks of every item: zero hidden states
     AR_CUDA_OK(cudaMemset2DAsync(h.h() + (long long)HALO * 8, (size_t)h.Tp * 16, 0, (size_t)w.lstm_start * 16, (size_t)B * 8, c.stream));
-  if (w.state_pos < T) {
+  if (w.cap != nullptr) {
+    AR_CHECK(state_out != nullptr, AR_ERR_INVALID, "stereo: per-item state positions need state_out");
+    AR_TRY(scan(w.lstm_start, T, state_in, state_out, w.cap));
+  } else if (w.state_pos < T) {
     AR_CHECK(state_out != nullptr, AR_ERR_INVALID, "stereo: an interior state_pos needs state_out");
     AR_TRY(scan(w.lstm_start, w.state_pos, state_in, state_out));
     AR_TRY(scan(w.state_pos, T, state_out, nullptr));
@@ -1050,17 +1055,20 @@ static int dispatch(Ctx& c, const float* x, float* y, int T, const float* st_in,
   return AR_ERR_INVALID;
 }
 
+// A stereo forward's workspace ends with room for B per-item LSTM state positions (ar_stereo_forward_window_multi)
+static size_t cap_bytes(const Model* m, int B) { return m->kind == AR_MODEL_STEREO ? ((size_t)B * sizeof(int) + 255) / 256 * 256 : 0; }
+
 int model_workspace_bytes(const Model* m, int B, int T, size_t* bytes) {
   AR_CHECK(m && bytes && B >= 1 && T >= 1, AR_ERR_INVALID, "workspace_bytes: bad argument");
   Ctx c;
   c.m = m; c.B = B; c.ar.dry = true;
   AR_TRY(dispatch(c, nullptr, nullptr, T, nullptr, nullptr));
-  *bytes = c.ar.peak + 256;
+  *bytes = c.ar.peak + 256 + cap_bytes(m, B);
   return AR_OK;
 }
 
 int model_forward(const Model* m, const float* x, float* y, int B, int T, const float* st_in, float* st_out, void* ws,
-                  size_t ws_bytes, cudaStream_t stream, int lstm_start, int state_pos) {
+                  size_t ws_bytes, cudaStream_t stream, int lstm_start, int state_pos, const int* state_pos_host) {
   AR_CHECK(m && x && y && B >= 1 && T >= 1, AR_ERR_INVALID, "forward: bad argument");
   size_t need = 0;
   AR_TRY(model_workspace_bytes(m, B, T, &need));
@@ -1070,10 +1078,25 @@ int model_forward(const Model* m, const float* x, float* y, int B, int T, const 
   c.ar.dry = false;
   uintptr_t a = (reinterpret_cast<uintptr_t>(ws) + 255) / 256 * 256;
   c.ar.base = reinterpret_cast<char*>(a);
-  c.ar.cap = need - 256;        // == the dry-run peak: high-side tensors are placed down from it
+  c.ar.cap = need - 256 - cap_bytes(m, B);   // == the dry-run peak: high-side tensors are placed down from it
   LstmWindow w;
   w.lstm_start = lstm_start;
   w.state_pos = state_pos;
+  if (state_pos_host != nullptr) {
+    AR_CHECK(m->kind == AR_MODEL_STEREO && st_out != nullptr, AR_ERR_INVALID, "forward: per-item state positions need a stereo model and state_out");
+    std::vector<int> local(B);
+    for (int b = 0; b < B; ++b) {
+      AR_CHECK(lstm_start < state_pos_host[b] && state_pos_host[b] <= T, AR_ERR_INVALID,
+               "stereo: state_pos[" + std::to_string(b) + "] = " + std::to_string(state_pos_host[b]) +
+                   " must satisfy lstm_start < state_pos <= T");
+      local[b] = state_pos_host[b] - lstm_start;   // the scan kernels count steps from lstm_start
+    }
+    int* dcap = reinterpret_cast<int*>(c.ar.base + c.ar.cap);
+    // pageable source: staged before the call returns, so `local` may go; no host sync
+    AR_CUDA_OK(cudaMemcpyAsync(dcap, local.data(), (size_t)B * sizeof(int), cudaMemcpyHostToDevice, stream));
+    w.cap = dcap;
+    w.state_pos = T;
+  }
   return dispatch(c, x, y, T, st_in, st_out, w);
 }
 

@@ -2,6 +2,9 @@
 // denoiser mask logic and the super-res linear-interp residual), normalize, chunk split and
 // overlap-add.  All are HBM-bound streaming passes with coalesced (float4 where the layout
 // allows) accesses.
+#include <cstring>
+#include <vector>
+
 #include "ar_common.cuh"
 #include "pointwise.cuh"
 
@@ -500,6 +503,68 @@ int launch_ola(const float* y, float* out, long long n, int n_chunks, int channe
     dim3 grid((unsigned)(want > 2368 ? 2368 : want), channels);
     ola_kernel<<<grid, 256, 0, stream>>>(y, out, n_out, n_chunks, channels, L, H, V, invV);
   }
+  AR_CUDA_OK(cudaGetLastError());
+  return AR_OK;
+}
+
+// ============================================================================ window gather / kept-range scatter
+// The lockstep whole-file-exact mode reads one window per file at a per-file offset of the stage-1 signals and writes one
+// kept range per file back: one launch each way for all files of a step instead of one copy per file.
+__global__ void gather_windows_kernel(const float* __restrict__ src, const long long* __restrict__ off, int W, float* __restrict__ dst) {
+  const int b = blockIdx.y;
+  const float* s = src + off[b];
+  float* d = dst + (long long)b * W;
+  for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < W; j += gridDim.x * blockDim.x) d[j] = s[j];
+}
+
+__global__ void scatter_kept_kernel(const float* __restrict__ y, int W, const long long* __restrict__ dst_off,
+                                    const int* __restrict__ lo, const int* __restrict__ len, float* __restrict__ out) {
+  const int b = blockIdx.y, ch = blockIdx.z;
+  const float* s = y + ((long long)b * 2 + ch) * W + lo[b];
+  float* d = out + dst_off[2 * b + ch];
+  const int n = len[b];
+  for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < n; j += gridDim.x * blockDim.x) d[j] = s[j];
+}
+
+static int window_grid(int W) { return (W + 1023) / 1024 < 64 ? (W + 1023) / 1024 : 64; }
+
+int launch_gather_windows(const float* src, long long src_len, const long long* offsets, int B, int W, float* dst, void* ws,
+                          size_t ws_bytes, cudaStream_t stream) {
+  AR_CHECK(src && offsets && dst && B >= 1 && W >= 1, AR_ERR_INVALID, "gather_windows: bad argument");
+  AR_CHECK(ws != nullptr && ws_bytes >= (size_t)B * AR_WINDOW_IO_BYTES_PER_ITEM, AR_ERR_WORKSPACE, "gather_windows: workspace too small");
+  for (int b = 0; b < B; ++b)
+    AR_CHECK(offsets[b] >= 0 && offsets[b] + W <= src_len, AR_ERR_INVALID,
+             "gather_windows: window " + std::to_string(b) + " at " + std::to_string(offsets[b]) + " leaves the source");
+  long long* d_off = reinterpret_cast<long long*>(ws);
+  AR_CUDA_OK(cudaMemcpyAsync(d_off, offsets, (size_t)B * sizeof(long long), cudaMemcpyHostToDevice, stream));
+  gather_windows_kernel<<<dim3(window_grid(W), B), 256, 0, stream>>>(src, d_off, W, dst);
+  AR_CUDA_OK(cudaGetLastError());
+  return AR_OK;
+}
+
+int launch_scatter_kept(const float* y, int B, int W, const long long* dst_offsets, const int* lo, const int* len, float* out,
+                        long long out_len, void* ws, size_t ws_bytes, cudaStream_t stream) {
+  AR_CHECK(y && dst_offsets && lo && len && out && B >= 1 && W >= 1, AR_ERR_INVALID, "scatter_kept: bad argument");
+  AR_CHECK(ws != nullptr && ws_bytes >= (size_t)B * AR_WINDOW_IO_BYTES_PER_ITEM, AR_ERR_WORKSPACE, "scatter_kept: workspace too small");
+  int max_len = 0;
+  for (int b = 0; b < B; ++b) {
+    AR_CHECK(lo[b] >= 0 && len[b] >= 0 && lo[b] + len[b] <= W, AR_ERR_INVALID, "scatter_kept: kept range " + std::to_string(b) + " leaves its window");
+    for (int ch = 0; ch < 2; ++ch)
+      AR_CHECK(dst_offsets[2 * b + ch] >= 0 && dst_offsets[2 * b + ch] + len[b] <= out_len, AR_ERR_INVALID,
+               "scatter_kept: kept range " + std::to_string(b) + " leaves the output");
+    max_len = len[b] > max_len ? len[b] : max_len;
+  }
+  // one upload: [B][2] offsets, then lo[B], len[B]
+  std::vector<char> stage((size_t)B * AR_WINDOW_IO_BYTES_PER_ITEM);
+  memcpy(stage.data(), dst_offsets, (size_t)B * 16);
+  memcpy(stage.data() + (size_t)B * 16, lo, (size_t)B * 4);
+  memcpy(stage.data() + (size_t)B * 20, len, (size_t)B * 4);
+  char* d = reinterpret_cast<char*>(ws);
+  AR_CUDA_OK(cudaMemcpyAsync(d, stage.data(), stage.size(), cudaMemcpyHostToDevice, stream));   // pageable: staged on return
+  if (max_len == 0) return AR_OK;
+  scatter_kept_kernel<<<dim3(window_grid(max_len), B, 2), 256, 0, stream>>>(
+      y, W, reinterpret_cast<const long long*>(d), reinterpret_cast<const int*>(d + (size_t)B * 16),
+      reinterpret_cast<const int*>(d + (size_t)B * 20), out);
   AR_CUDA_OK(cudaGetLastError());
   return AR_OK;
 }

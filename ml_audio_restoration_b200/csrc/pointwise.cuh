@@ -49,13 +49,19 @@ int launch_audit_tap(const Act& a, int B, int coff8, int nch8, int T, int tblock
 int launch_plain_to_c4(const float* x, int B, int C, int T, const Act& out, cudaStream_t stream);
 int launch_c4_to_plain(const Act& in, int B, int C, int T, float* y, cudaStream_t stream);
 
+int launch_gather_windows(const float* src, long long src_len, const long long* offsets, int B, int W, float* dst, void* ws,
+                          size_t ws_bytes, cudaStream_t stream);
+int launch_scatter_kept(const float* y, int B, int W, const long long* dst_offsets, const int* lo, const int* len, float* out,
+                        long long out_len, void* ws, size_t ws_bytes, cudaStream_t stream);
+
 // xp: H8 fp16 [B][256 ch] gate pre-activations (W_ih x + b_ih + b_hh, rows i|f|g|o), whh: [256][64] device,
-// h_out: H8 fp16 [B][64 ch]; state_in/out: [B][2][64] (h, c) or nullptr.
+// h_out: H8 fp16 [B][64 ch]; state_in/out: [B][2][64] (h, c) or nullptr.  cap: nullptr (state_out after the last step) or
+// a device array [B]: sequence b writes state_out[b] after step cap[b] - 1 (cap[b] >= T: the last) and runs on.
 int launch_lstm(const Act& xp, const float* whh, const Act& h_out, int B, int T, const float* state_in, float* state_out,
-                cudaStream_t stream);
+                const int* cap, cudaStream_t stream);
 // scan that computes its own input projection on the tensor pipe (lstm_proj.cu): x = encoder output, 128 channels
 void pack_lstm_proj(const float* G, std::vector<uint16_t>& out);
 int launch_lstm_proj(const Act& x, const __half* wih_packed, const float* bias, const float* whh, const Act& h_out, int B, int T,
-                     const float* state_in, float* state_out, cudaStream_t stream);
+                     const float* state_in, float* state_out, const int* cap, cudaStream_t stream);
 
 }  // namespace ar

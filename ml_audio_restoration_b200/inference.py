@@ -52,6 +52,32 @@ def plan_chunks(num_samples: int, chunk_size: int = DEFAULT_CHUNK, overlap: int 
     return [i * hop for i in range(n)]
 
 
+def plan_exact_windows(M: int, S: int, E: int = EXACT_STEREO_HALO, P: int = EXACT_LSTM_LEAD):
+    """Stereo-stage segmentation of one file of `M` samples for the lockstep whole-file-exact mode (`restore_many`):
+    every window is `W = S + 2E` samples long and lies inside `[0, M)`, so the windows of many files form uniform
+    launches.  Returns `[(start, lstm_start, keep_lo, keep_hi, state_pos)]` in window coordinates (the window is
+    `[start, start + W)` of the file, it keeps `[start + keep_lo, start + keep_hi)`), or None when `M < W` (the file runs
+    alone through `restore`).
+
+    With `n >= 2` windows and `k = M - E - (n - 1) S`, `E <= k <= S + E`: the first window `[0, W)` keeps `[0, k)` and
+    hands its state on at `k - P`, the only position that differs between files; interior windows start `E` before
+    their kept range of `S` samples, scan from `E - P` and hand on at `S + E - P`; the last window `[M - W, M)` keeps its
+    last `S + E` samples, so it ends at the file end without padding.  Each hand-on position is where the next window's
+    scan starts, and at least `E + P` samples before its window's right edge: the LSTM inputs there are exact."""
+    W = S + 2 * E
+    if M < W:
+        return None
+    n1 = max(1, -(-(M - W) // S))                   # n - 1
+    k = M - E - n1 * S
+    wins = [(0, 0, 0, k, k - P)]
+    for j in range(1, n1 + 1):
+        a0 = k + (j - 1) * S
+        last = j == n1
+        start = M - W if last else a0 - E
+        wins.append((start, E - P, E, E + S + (E if last else 0), S + E - P))
+    return wins
+
+
 def shard_range(n_items: int, rank: int, world: int):
     """Contiguous block partition `[lo, hi)` of chunk (or file) indices for one GPU (SURVEY.md 8e)."""
     lo = n_items * rank // world
@@ -308,14 +334,266 @@ class RestorationPipeline:
             ev.synchronize()
             yield h
 
+    @torch.no_grad()
+    def restore_many(self, audios, mode: str = "chunked", chunk_size: int = DEFAULT_CHUNK, overlap: int = DEFAULT_OVERLAP,
+                     batch_chunks: int = 0, normalize: bool = True, return_device: bool = False, **excluded) -> list:
+        """Many mono files (`[1,N]` or `[N]`, host or device) -> their restored stereo `[2, rate*N]`, in input order.
+
+        Each result is what `restore(audio, mode=mode, ...)` returns for that file (bitwise where the same kernel
+        instances run, else within the tolerance between the LSTM kernels), but the files share chain launches, so a
+        catalog of short sides fills the GPU like one long file does:
+
+        * `mode="chunked"`: the chunks of a group of files form ONE `forward_chunks` batch (up to 16 per SM, the
+          `auto_batch` rule); split, overlap-add and normalisation run per file on its own slice.  A file with more
+          chunks than a group holds runs alone.
+        * `mode="exact"`: stage 1 (denoise -> super-res) runs the full chunks of all files of a group in shared
+          batches; the stereo stage runs the files in lockstep, window j of every file in ONE `forward_window` launch
+          with per-file state positions (`plan_exact_windows`), the LSTM state passed from step to step.  Files
+          shorter than one window run alone.
+
+        `normalize` applies per file, as in `restore`."""
+        for key in ("chunk_range", "reuse_output", "streams"):
+            if key in excluded:
+                raise ValueError(f"restore_many does not take {key}")
+        if excluded:
+            raise TypeError(f"restore_many got unexpected arguments {sorted(excluded)}")
+        if mode not in ("chunked", "exact"):
+            raise ValueError(f"restore_many: mode must be 'chunked' or 'exact', got {mode!r}")
+        audios = list(audios)
+        if not audios:
+            return []
+        was_host = []
+        files = []
+        with torch.cuda.device(self.device):
+            for audio in audios:
+                if audio.dim() == 1:
+                    audio = audio.unsqueeze(0)
+                if audio.dim() != 2 or audio.shape[0] != 1:
+                    raise RuntimeError(f"expected mono audio [1, N], got {tuple(audio.shape)}")
+                if audio.shape[1] == 0:
+                    raise ValueError("empty audio")
+                was_host.append(not audio.is_cuda)
+                files.append(audio)
+            run = self._many_chunked if mode == "chunked" else self._many_exact
+            outs = run(files, chunk_size, overlap, batch_chunks, normalize)
+        return [y.cpu() if h and not return_device else y for y, h in zip(outs, was_host)]
+
+    def _prepared(self, audio, normalize):
+        """Device copy of one mono file, normalised like `restore` normalises it."""
+        a = audio.to(self.device, torch.float32, non_blocking=True).contiguous()
+        if a.data_ptr() == audio.data_ptr():
+            a = a.clone()
+        if normalize:
+            self._normalize_(a)
+        return a
+
+    def _budget(self):
+        free, _ = torch.cuda.mem_get_info(self.device)
+        held = sum(b.numel() for b in (self._ws or {}).values() if b is not None)
+        return int((free + held) * 0.85)
+
+    @staticmethod
+    def _packed(sizes, device):
+        """One buffer holding tensors of `sizes` floats, each starting on a 16-byte boundary (`ar_normalize` needs it)."""
+        offs, total = [], 0
+        for n in sizes:
+            offs.append(total)
+            total += -(-n // 4) * 4
+        return torch.empty(max(total, 1), dtype=torch.float32, device=device), offs
+
+    def _many_chunked(self, files, chunk_size, overlap, batch_chunks, normalize):
+        r, L = self.rate, _lib.lib()
+        counts = [len(plan_chunks(a.shape[1], chunk_size, overlap)) for a in files]
+        if batch_chunks <= 0:
+            batch_chunks = self.auto_batch(sum(counts), chunk_size)
+        # the workspace of a full group up front: groups of slightly different sizes then share one buffer instead of
+        # growing it while the previous one is still referenced
+        self._workspace(self.workspace_bytes(min(batch_chunks, sum(counts)), chunk_size))
+        outs = [None] * len(files)
+        group = []
+
+        def flush():
+            if not group:
+                return
+            total = sum(counts[f] for f in group)
+            buf = torch.empty((total, 1, chunk_size), dtype=torch.float32, device=self.device)
+            first = 0
+            for f in group:
+                a = self._prepared(files[f], normalize)
+                _lib.check(L.ar_split_chunks(a.data_ptr(), a.shape[1], buf[first].data_ptr(), 0, counts[f], chunk_size, overlap,
+                                             self._stream()))
+                first += counts[f]
+            y_all = self.forward_chunks(buf)
+            out, offs = self._packed([2 * r * files[f].shape[1] for f in group], self.device)
+            first = 0
+            for f, o in zip(group, offs):
+                N = files[f].shape[1]
+                y = out[o:o + 2 * r * N].view(2, r * N)
+                _lib.check(L.ar_overlap_add(y_all[first].data_ptr(), y.data_ptr(), N, counts[f], 2, chunk_size, overlap, r,
+                                            self._stream()))
+                if normalize:
+                    self._normalize_(y)
+                outs[f] = y
+                first += counts[f]
+            group.clear()
+
+        for f in range(len(files)):
+            if counts[f] > batch_chunks:                     # larger than a group: alone, as `restore` runs it
+                outs[f] = self.restore(files[f], mode="chunked", chunk_size=chunk_size, overlap=overlap,
+                                       batch_chunks=batch_chunks, normalize=normalize, return_device=True)
+                continue
+            if sum(counts[g] for g in group) + counts[f] > batch_chunks:
+                flush()
+            group.append(f)
+        flush()
+        return outs
+
+    def _many_exact(self, files, chunk_size, overlap, batch_chunks, normalize):
+        r, E, P = self.rate, EXACT_STEREO_HALO, EXACT_LSTM_LEAD
+        Lc = chunk_size - chunk_size % 8
+        if Lc < 4 * EXACT_HALO:
+            raise ValueError(f"mode='exact' needs chunk_size >= {4 * EXACT_HALO} (conv halos of {EXACT_HALO} samples per chunk edge)")
+        S = (r * Lc - 2 * E) // 16 * 16
+        W = S + 2 * E
+        outs = [None] * len(files)
+        plans = [plan_exact_windows(r * a.shape[1], S) for a in files]
+        lock = []
+        for f, plan in enumerate(plans):
+            if plan is None:                                 # shorter than one window: alone
+                outs[f] = self.restore(files[f], mode="exact", chunk_size=chunk_size, batch_chunks=batch_chunks,
+                                       normalize=normalize, return_device=True)
+            else:
+                lock.append(f)
+        if not lock:
+            return outs
+        # groups: up to 16 windows per SM (8, then whatever fits) beside the files' stage-1 signals and outputs
+        sms = torch.cuda.get_device_properties(self.device).multi_processor_count
+        budget = self._budget()
+        per_file = lambda f: 4 * 3 * r * files[f].shape[1]  # stage-1 signal + stereo output
+        cap = 1
+        for per_sm in (16, 8, 2):
+            cap = min(len(lock), per_sm * sms)
+            if self.stereo_workspace_bytes(cap, W) <= budget // 2:
+                break
+        groups, cur, used = [], [], 0
+        for f in lock:
+            if cur and (len(cur) == cap or used + per_file(f) > budget // 2):
+                groups.append(cur)
+                cur, used = [], 0
+            cur.append(f)
+            used += per_file(f)
+        groups.append(cur)
+        for grp in groups:
+            self._exact_group([files[f] for f in grp], [plans[f] for f in grp], Lc, W, batch_chunks, normalize,
+                              outs, grp)
+        return outs
+
+    def stereo_workspace_bytes(self, batch: int, T: int) -> int:
+        need = C.c_size_t()
+        with torch.cuda.device(self.device):
+            _lib.check(_lib.lib().ar_model_workspace_bytes(self.stereo.native_handle(self.device), batch, T, C.byref(need)))
+        return need.value
+
+    def _exact_group(self, files, plans, Lc, W, batch_chunks, normalize, outs, idx):
+        r, L = self.rate, _lib.lib()
+        Ns = [a.shape[1] for a in files]
+        Ms = [r * n for n in Ns]
+        sig_all, sig_offs = self._packed(Ms, self.device)
+        out_all, out_offs = self._packed([2 * m for m in Ms], self.device)
+        ins = [self._prepared(a, normalize) for a in files]
+        self._exact_stage1(ins, [sig_all[o:o + m].view(1, m) for o, m in zip(sig_offs, Ms)], Lc, batch_chunks)
+        # lockstep over windows: files sorted by window count, so the files still running at step j are a prefix and
+        # the state of step j + 1 is the first rows of the state step j returned
+        order = sorted(range(len(files)), key=lambda i: -len(plans[i]))
+        ws = torch.empty(_lib.WINDOW_IO_BYTES_PER_ITEM * len(files), dtype=torch.uint8, device=self.device)
+        state = None
+        for j in range(len(plans[order[0]])):
+            act = [i for i in order if len(plans[i]) > j]
+            B = len(act)
+            wins = [plans[i][j] for i in act]
+            x = torch.empty((B, 1, W), dtype=torch.float32, device=self.device)
+            offs = (C.c_int64 * B)(*[sig_offs[i] + w[0] for i, w in zip(act, wins)])
+            _lib.check(L.ar_gather_windows(sig_all.data_ptr(), sig_all.numel(), offs, B, W, x.data_ptr(), ws.data_ptr(),
+                                           ws.numel(), self._stream()))
+            y, state = self.stereo.forward_window(x, None if state is None else state[:B], lstm_start=wins[0][1],
+                                                  state_pos=[w[4] for w in wins])
+            dst = []
+            for i, w in zip(act, wins):
+                dst += [out_offs[i] + w[0] + w[2], out_offs[i] + Ms[i] + w[0] + w[2]]
+            _lib.check(L.ar_scatter_kept(y.data_ptr(), B, W, (C.c_int64 * (2 * B))(*dst), (C.c_int * B)(*[w[2] for w in wins]),
+                                         (C.c_int * B)(*[w[3] - w[2] for w in wins]), out_all.data_ptr(), out_all.numel(),
+                                         ws.data_ptr(), ws.numel(), self._stream()))
+        for i, (o, m) in enumerate(zip(out_offs, Ms)):
+            y = out_all[o:o + 2 * m].view(2, m)
+            if normalize:
+                self._normalize_(y)
+            outs[idx[i]] = y
+
+    def _exact_stage1(self, ins, sigs, L, batch_chunks):
+        """Stage 1 of the whole-file-exact mode (denoise -> super-res) for normalised mono `[1,N]` device signals `ins`
+        into `sigs[f]` (`[1, rate*N]`).  Chunk i of a file covers input samples `[i*hop, i*hop + L)` with
+        `hop = L - 2*EXACT_HALO`; the full chunks of all files run as shared batches, a ragged tail chunk runs alone at
+        its true length (zero-padding it would move the file end), and only the samples further than EXACT_HALO from
+        an interior chunk edge are kept.  Chunk starts are multiples of 8, so every chunk sees the pooling grid of the
+        whole file (SURVEY.md App. E)."""
+        r, H = self.rate, EXACT_HALO
+        hop = L - 2 * H
+        lib = _lib.lib()
+
+        def stage1(x):                                  # [B,1,T] -> [B,1,r*T]
+            y = self.denoiser(x)
+            return self.super_res(y) if self.super_res is not None else y
+
+        plans = []
+        for a in ins:
+            N = a.shape[1]
+            n = 1 if N <= L else -(-(N - 2 * H) // hop)
+            plans.append((N, n, n if (n - 1) * hop + L <= N else n - 1))
+        full = [(f, i) for f, (_, _, n_full) in enumerate(plans) for i in range(n_full)]
+        if batch_chunks <= 0:
+            free, _ = torch.cuda.mem_get_info(self.device)
+            sms = torch.cuda.get_device_properties(self.device).multi_processor_count
+            batch_chunks = max(1, min(len(full), 8 * sms, self.max_batch(L, int(free * 0.5))))
+        for b0 in range(0, len(full), batch_chunks):
+            items = full[b0:b0 + batch_chunks]
+            buf = torch.empty((len(items), 1, L), dtype=torch.float32, device=self.device)
+            runs = []                                   # (file, first chunk, count, batch row) of each file in this batch
+            for row, (f, i) in enumerate(items):
+                if runs and runs[-1][0] == f:
+                    runs[-1][2] += 1
+                else:
+                    runs.append([f, i, 1, row])
+            for f, first, cnt, row in runs:
+                a = ins[f]
+                _lib.check(lib.ar_split_chunks(a.data_ptr(), a.shape[1], buf[row].data_ptr(), first, cnt, L, 2 * H, self._stream()))
+            z_all = stage1(buf)
+            for f, first, cnt, row in runs:
+                N, n, _ = plans[f]
+                sig, z = sigs[f], z_all[row:row + cnt]
+
+                def keep(i):                            # kept input range of chunk i
+                    return 0 if i == 0 else i * hop + H, N if i == n - 1 else (i + 1) * hop + H
+
+                for i in range(first, first + cnt):
+                    if i == 0 or i == n - 1:            # file edges keep their outer side
+                        lo, hi = keep(i)
+                        sig[:, r * lo:r * hi] = z[i - first, :, r * (lo - i * hop):r * (hi - i * hop)]
+                i0, i1 = max(first, 1), min(first + cnt, n - 1)     # interior chunks: one strided copy
+                if i1 > i0:
+                    lo = i0 * hop + H
+                    sig[0, r * lo:r * (lo + (i1 - i0) * hop)].view(i1 - i0, r * hop).copy_(
+                        z[i0 - first:i1 - first, 0, r * H:r * (H + hop)])
+        for f, (N, n, n_full) in enumerate(plans):
+            if n_full < n:                              # ragged tail chunk at its true length
+                start = (n - 1) * hop
+                lo = 0 if n == 1 else (n - 1) * hop + H
+                z = stage1(ins[f][:, start:N].reshape(1, 1, N - start).contiguous())
+                sigs[f][:, r * lo:r * N] = z[0, :, r * (lo - start):r * (N - start)]
+
     def _restore_exact(self, a, N, chunk_size, batch_chunks):
         """Whole-file-exact chunked restoration of a normalised mono `[1,N]` device signal -> `[2, rate*N]`.
 
-        Stage 1, denoise (-> super-res): chunk i covers input samples `[i*hop, i*hop + L)` with `L = chunk_size` rounded
-        down to a multiple of 8 and `hop = L - 2*EXACT_HALO`; all full chunks run as batches, a ragged tail chunk runs
-        alone at its true length (zero-padding it would move the file end), and only the samples further than
-        EXACT_HALO from an interior chunk edge are kept.  Chunk starts are multiples of 8, so every chunk sees the
-        pooling grid of the whole file (SURVEY.md App. E).
+        Stage 1, denoise (-> super-res): `_exact_stage1` with `L = chunk_size` rounded down to a multiple of 8.
         Stage 2, stereo: segments of the stage-1 signal with EXACT_STEREO_HALO samples of context on both sides go
         through `forward_window` one after the other; the scan of segment j starts EXACT_LSTM_LEAD samples before the
         segment's kept range from the (h, c) its predecessor recorded at exactly that sample."""
@@ -323,43 +601,8 @@ class RestorationPipeline:
         L = chunk_size - chunk_size % 8
         if L < 4 * H:
             raise ValueError(f"mode='exact' needs chunk_size >= {4 * H} (conv halos of {H} samples per chunk edge)")
-        hop = L - 2 * H
-        lib = _lib.lib()
-        n = 1 if N <= L else -(-(N - 2 * H) // hop)
-        n_full = n if (n - 1) * hop + L <= N else n - 1
         sig = torch.empty((1, r * N), dtype=torch.float32, device=self.device)
-
-        def stage1(x):                                  # [B,1,T] -> [B,1,r*T]
-            y = self.denoiser(x)
-            return self.super_res(y) if self.super_res is not None else y
-
-        def keep(i):                                    # kept input range of chunk i
-            lo = 0 if i == 0 else i * hop + H
-            hi = N if i == n - 1 else (i + 1) * hop + H
-            return lo, hi
-
-        if batch_chunks <= 0:
-            free, _ = torch.cuda.mem_get_info(self.device)
-            sms = torch.cuda.get_device_properties(self.device).multi_processor_count
-            batch_chunks = max(1, min(n_full, 8 * sms, self.max_batch(L, int(free * 0.5))))
-        for first in range(0, n_full, batch_chunks):
-            cnt = min(batch_chunks, n_full - first)
-            buf = torch.empty((cnt, 1, L), dtype=torch.float32, device=self.device)
-            _lib.check(lib.ar_split_chunks(a.data_ptr(), N, buf.data_ptr(), first, cnt, L, 2 * H, self._stream()))
-            z = stage1(buf)
-            for i in range(first, first + cnt):
-                if i == 0 or i == n - 1:                # file edges keep their outer side
-                    lo, hi = keep(i)
-                    sig[:, r * lo:r * hi] = z[i - first, :, r * (lo - i * hop):r * (hi - i * hop)]
-            i0, i1 = max(first, 1), min(first + cnt, n - 1)     # interior chunks: one strided copy
-            if i1 > i0:
-                lo = i0 * hop + H
-                sig[0, r * lo:r * (lo + (i1 - i0) * hop)].view(i1 - i0, r * hop).copy_(z[i0 - first:i1 - first, 0, r * H:r * (H + hop)])
-        if n_full < n:                                  # ragged tail chunk at its true length
-            lo, hi = keep(n - 1)
-            start = (n - 1) * hop
-            z = stage1(a[:, start:N].reshape(1, 1, N - start).contiguous())
-            sig[:, r * lo:r * hi] = z[0, :, r * (lo - start):r * (hi - start)]
+        self._exact_stage1([a], [sig], L, batch_chunks)
 
         M, E, P = r * N, EXACT_STEREO_HALO, EXACT_LSTM_LEAD
         S2 = (r * L - 2 * E) // 16 * 16                 # kept samples per stereo segment
@@ -602,6 +845,9 @@ def restore_audio(
     """
     if torch.device(device).type != 'cuda':
         raise RuntimeError("restore_audio: device must be a CUDA device -- this build has no CPU fallback")
+    if os.path.isdir(input_path):
+        return _restore_directory(input_path, output_path, denoiser_checkpoint, super_res_checkpoint, stereo_checkpoint,
+                                  sample_rate, enable_super_resolution, device, mode, chunk_size, overlap, output_encoding)
     print(f"Processing: {input_path}")
     print(f"Device: {device}")
     print("Loading audio...")
@@ -633,10 +879,57 @@ def restore_audio(
     print(f"Output sample rate: {out_rate}Hz{suffix}")
 
 
+def _restore_directory(input_dir, output_dir, denoiser_checkpoint, super_res_checkpoint, stereo_checkpoint, sample_rate,
+                       enable_super_resolution, device, mode, chunk_size, overlap, output_encoding):
+    """`restore_audio` on a directory: every `*.wav` / `*.flac` directly inside `input_dir`, in sorted order, into
+    `output_dir` under the same file name and container.  Checkpoints load once and the files share chain launches
+    (`restore_many`): `mode='chunked'` packs their chunks, `'whole'` and `'exact'` run the lockstep whole-file-exact path.
+    Every file goes through the dynamic-range audit first; its share of the run time is printed."""
+    import time
+    names = sorted(n for n in os.listdir(input_dir)
+                   if os.path.isfile(os.path.join(input_dir, n)) and os.path.splitext(n)[1].lower() in (".wav", ".flac"))
+    print(f"Processing directory: {input_dir} ({len(names)} files)")
+    print(f"Device: {device}")
+    os.makedirs(output_dir, exist_ok=True)
+    print("Loading denoiser model...")
+    den = _load_checkpoint(AudioDenoiser(), denoiser_checkpoint, device)
+    sr = None
+    if enable_super_resolution:
+        print("Loading super-resolution model...")
+        sr = _load_checkpoint(AudioSuperResolution(upscale_factor=2), super_res_checkpoint, device)
+    print("Loading stereo separator model...")
+    st = _load_checkpoint(StereoSeparator(), stereo_checkpoint, device)
+    pipe = RestorationPipeline(den, sr, st, device)
+    t0 = time.perf_counter()
+    audios, t_audit = [], 0.0
+    for n in names:
+        print(f"Loading audio: {os.path.join(input_dir, n)}")
+        audio, _ = load_audio_cuda(os.path.join(input_dir, n), sample_rate=sample_rate, device=device)
+        torch.cuda.synchronize(pipe.device)
+        t = time.perf_counter()
+        pipe.check_dynamic_range(audio, chunk_size)   # raises if this checkpoint clips the fp16 activation storage
+        t_audit += time.perf_counter() - t
+        audios.append(audio)
+    print("Applying denoising, " + ("bandwidth extension (22.05kHz -> 44.1kHz), " if enable_super_resolution else "") +
+          "stereo separation...")
+    outs = pipe.restore_many(audios, mode="chunked" if mode == "chunked" else "exact", chunk_size=chunk_size,
+                             overlap=overlap, return_device=True)
+    out_rate = sample_rate * pipe.rate
+    for n, stereo in zip(names, outs):
+        print(f"Saving to: {os.path.join(output_dir, n)}")
+        save_audio(os.path.join(output_dir, n), stereo, out_rate, encoding=output_encoding)
+    torch.cuda.synchronize(pipe.device)
+    total = time.perf_counter() - t0
+    print(f"Dynamic-range audit: {t_audit:.2f} s of {total:.2f} s ({100 * t_audit / max(total, 1e-9):.0f} %)")
+    print("Restoration complete!")
+    suffix = " (bandwidth extended)" if enable_super_resolution else ""
+    print(f"Output sample rate: {out_rate}Hz{suffix}")
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser(description='Restore 78rpm record audio')
-    ap.add_argument('input', type=str, help='Input audio file path')
-    ap.add_argument('output', type=str, help='Output audio file path')
+    ap.add_argument('input', type=str, help='Input audio file path (a directory: every *.wav / *.flac directly inside it)')
+    ap.add_argument('output', type=str, help='Output audio file path (a directory when the input is one)')
     ap.add_argument('--denoiser', type=str, default='models/checkpoints/best_model.pth', help='Path to denoiser checkpoint')
     ap.add_argument('--super-res', type=str, default='models/checkpoints/super_resolution/best_model.pth',
                     help='Path to super-resolution checkpoint')

@@ -59,9 +59,17 @@ class StereoSeparator(NativeModule):
     def forward_window(self, x, state=None, lstm_start: int = 0, state_pos=None):
         """Forward on a window of a longer signal (`ar_stereo_forward_window`): convs over all of `x[B,1,T]`, the LSTM
         scan over steps `[lstm_start, T)` from `state` (None = zeros), returned state taken after step `state_pos - 1`
-        (None = T).  Building block of `RestorationPipeline.restore(mode="exact")`."""
+        (None = T).  `state_pos` may also be a sequence of B ints, `lstm_start < state_pos[b] <= T`: item b hands its
+        state on at its own step, in the same scan (`ar_stereo_forward_window_multi`).  Building block of
+        `RestorationPipeline.restore(mode="exact")` and `restore_many(mode="exact")`."""
         x = self._check_input(x)
         B, _, T = x.shape
+        per_item = state_pos is not None and not isinstance(state_pos, int)
+        if per_item:
+            pos = [int(p) for p in state_pos]
+            if len(pos) != B:
+                raise ValueError(f"state_pos has {len(pos)} entries for a batch of {B}")
+            pos = (C.c_int * B)(*pos)
         L = _lib.lib()
         with torch.cuda.device(x.device):
             h = self.native_handle(x.device)
@@ -75,8 +83,13 @@ class StereoSeparator(NativeModule):
                 sin = state.to(device=x.device, dtype=torch.float32).contiguous()
                 if sin.shape != new_state.shape:
                     raise RuntimeError(f"state must be {tuple(new_state.shape)}, got {tuple(sin.shape)}")
-            _lib.check(L.ar_stereo_forward_window(h, x.data_ptr(), y.data_ptr(), B, T, int(lstm_start),
-                                                  T if state_pos is None else int(state_pos),
-                                                  sin.data_ptr() if sin is not None else None, new_state.data_ptr(),
-                                                  ws.data_ptr(), ws.numel(), _stream_ptr(x.device)))
+            sin_ptr = sin.data_ptr() if sin is not None else None
+            if per_item:
+                _lib.check(L.ar_stereo_forward_window_multi(h, x.data_ptr(), y.data_ptr(), B, T, int(lstm_start), pos, sin_ptr,
+                                                            new_state.data_ptr(), ws.data_ptr(), ws.numel(),
+                                                            _stream_ptr(x.device)))
+            else:
+                _lib.check(L.ar_stereo_forward_window(h, x.data_ptr(), y.data_ptr(), B, T, int(lstm_start),
+                                                      T if state_pos is None else int(state_pos), sin_ptr,
+                                                      new_state.data_ptr(), ws.data_ptr(), ws.numel(), _stream_ptr(x.device)))
         return y, new_state
