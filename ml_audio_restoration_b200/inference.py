@@ -13,7 +13,7 @@ Two ways through the same three native models:
   shard across GPUs with no collective.
 * exact (`mode="exact"`, SURVEY.md 8f n2): chunked, but equal to the whole-file result: chunk starts are multiples of 8
   (the U-Net's three pools), every chunk carries conv halos that are computed and discarded, and the stereo LSTM's
-  (h, c) is carried from segment to segment of the file, so the scan is the reference's single scan
+  (h, c) is carried from window to window of the file, so the scan is the reference's single scan
   (stereo_separator.py:106-107).  Bounded memory for files of any length; the scan of one file is serial.
 """
 from __future__ import annotations
@@ -53,11 +53,11 @@ def plan_chunks(num_samples: int, chunk_size: int = DEFAULT_CHUNK, overlap: int 
 
 
 def plan_exact_windows(M: int, S: int, E: int = EXACT_STEREO_HALO, P: int = EXACT_LSTM_LEAD):
-    """Stereo-stage segmentation of one file of `M` samples for the lockstep whole-file-exact mode (`restore_many`):
+    """Stereo-stage segmentation of one file of `M` samples for the whole-file-exact mode (`restore` and `restore_many`):
     every window is `W = S + 2E` samples long and lies inside `[0, M)`, so the windows of many files form uniform
     launches.  Returns `[(start, lstm_start, keep_lo, keep_hi, state_pos)]` in window coordinates (the window is
     `[start, start + W)` of the file, it keeps `[start + keep_lo, start + keep_hi)`), or None when `M < W` (the file runs
-    alone through `restore`).
+    through one stereo forward over its whole signal).
 
     With `n >= 2` windows and `k = M - E - (n - 1) S`, `E <= k <= S + E`: the first window `[0, W)` keeps `[0, k)` and
     hands its state on at `k - P`, the only position that differs between files; interior windows start `E` before
@@ -85,10 +85,34 @@ def shard_range(n_items: int, rank: int, world: int):
     return lo, hi
 
 
+def _as_mono(audio: torch.Tensor) -> torch.Tensor:
+    """`[N]` or `[1, N]` mono audio as `[1, N]`; anything else, or no samples, is refused."""
+    if audio.dim() == 1:
+        audio = audio.unsqueeze(0)
+    if audio.dim() != 2 or audio.shape[0] != 1:
+        raise RuntimeError(f"expected mono audio [1, N], got {tuple(audio.shape)}")
+    if audio.shape[1] == 0:
+        raise ValueError("empty audio")
+    return audio
+
+
 def _load_checkpoint(module, path, device):
     ckpt = torch.load(path, map_location="cpu")
     module.load_state_dict(ckpt["model_state_dict"])
     return module.to(device).eval()
+
+
+def _load_pipeline(denoiser_checkpoint, super_res_checkpoint, stereo_checkpoint, enable_super_resolution, device):
+    """The `RestorationPipeline` of three checkpoint files, with `restore_audio`'s progress prints."""
+    print("Loading denoiser model...")
+    den = _load_checkpoint(AudioDenoiser(), denoiser_checkpoint, device)
+    sr = None
+    if enable_super_resolution:
+        print("Loading super-resolution model...")
+        sr = _load_checkpoint(AudioSuperResolution(upscale_factor=2), super_res_checkpoint, device)
+    print("Loading stereo separator model...")
+    st = _load_checkpoint(StereoSeparator(), stereo_checkpoint, device)
+    return RestorationPipeline(den, sr, st, device)
 
 
 class RestorationPipeline:
@@ -193,17 +217,45 @@ class RestorationPipeline:
         return need.value
 
     def max_batch(self, chunk_size: int, budget_bytes: int) -> int:
-        """Largest chunk batch (up to 8 per SM) whose chain workspace fits in `budget_bytes`."""
+        """Largest chunk batch (at least 1) whose chain workspace, at one chunk's workspace per chunk, fits in
+        `budget_bytes`."""
         return max(1, int(budget_bytes // max(1, self.workspace_bytes(1, chunk_size))))
+
+    # ------------------------------------------------------------------ memory rules
+    def _memory(self):
+        """(free device bytes, bytes of the workspaces this pipeline caches, SM count): what the rules below size from."""
+        free, _ = torch.cuda.mem_get_info(self.device)
+        held = sum(b.numel() for b in (self._ws or {}).values() if b is not None)
+        return free, held, torch.cuda.get_device_properties(self.device).multi_processor_count
+
+    @staticmethod
+    def _budget(free: int, held: int) -> int:
+        """Bytes the launches of one call may use: 85 % of the free memory, counting the cached workspaces (they get
+        reused)."""
+        return int((free + held) * 0.85)
+
+    @staticmethod
+    def _stage1_batch(n_chunks: int, free: int, sms: int, chunk_ws: int) -> int:
+        """Chunks per stage-1 launch of the exact mode: up to 8 per SM, as many as fit in half the free memory at
+        `chunk_ws` bytes of chain workspace per chunk."""
+        return max(1, min(n_chunks, 8 * sms, max(1, int(free * 0.5) // max(1, chunk_ws))))
+
+    @staticmethod
+    def _group_cap(n_files: int, budget: int, sms: int, stereo_ws) -> int:
+        """Files per lockstep group of the exact mode: 16 windows per SM, else 8, else 2, the first whose stereo workspace
+        (`stereo_ws(batch)` bytes) fits in half the budget; 2 per SM when none does."""
+        for per_sm in (16, 8, 2):
+            cap = min(n_files, per_sm * sms)
+            if stereo_ws(cap) <= budget // 2:
+                break
+        return cap
 
     def auto_batch(self, n_chunks: int, chunk_size: int, streams: int = 1) -> int:
         """Chunks per chain launch.  16 per SM when the workspace allows it (one tensor-core LSTM scan, 8 sequences per CTA,
         two CTAs per SM, fills the chip; the chain runs its conv phases on sub-batches around it), else 8 per SM (4 per
         CTA), else whatever fits."""
-        free, _ = torch.cuda.mem_get_info(self.device)
-        held = sum(b.numel() for b in (self._ws or {}).values() if b is not None)     # cached workspaces get reused
-        budget = int((free + held) * 0.85) // max(1, streams)
-        sms = torch.cuda.get_device_properties(self.device).multi_processor_count
+        free, held, sms = self._memory()
+        budget = self._budget(free, held) // max(1, streams)
         for per_sm in (16, 8):
             if n_chunks > (per_sm // 2) * sms and self.workspace_bytes(min(n_chunks, per_sm * sms), chunk_size) <= budget:
                 return min(n_chunks, per_sm * sms)
@@ -224,22 +276,13 @@ class RestorationPipeline:
         unsharded result.  Sharded calls need `normalize=False`: `normalize_audio` is global, so the
         caller normalises the input first and the concatenated output afterwards.
         """
-        if audio.dim() == 1:
-            audio = audio.unsqueeze(0)
-        if audio.dim() != 2 or audio.shape[0] != 1:
-            raise RuntimeError(f"expected mono audio [1, N], got {tuple(audio.shape)}")
+        audio = _as_mono(audio)
         N = audio.shape[1]
-        if N == 0:
-            raise ValueError("empty audio")
         if chunk_range is not None and normalize:
             raise ValueError("chunk_range needs normalize=False (normalisation is global over the file)")
         was_host = not audio.is_cuda
         with torch.cuda.device(self.device):
-            a = audio.to(self.device, torch.float32, non_blocking=True).contiguous()
-            if a.data_ptr() == audio.data_ptr():
-                a = a.clone()
-            if normalize:
-                self._normalize_(a)
+            a = self._prepared(audio, normalize)
             if mode == "auto":
                 mode = "whole" if N <= chunk_size else "chunked"
             if mode == "whole":
@@ -249,7 +292,7 @@ class RestorationPipeline:
             elif mode == "exact":
                 if chunk_range is not None:
                     raise ValueError("mode='exact' carries the LSTM state through the file: it cannot be sharded by chunk range")
-                y = self._restore_exact(a, N, chunk_size, batch_chunks)
+                y = self._restore_exact([a], chunk_size, batch_chunks)[0]
             else:
                 raise ValueError(f"unknown mode {mode!r}")
             if normalize:
@@ -288,13 +331,8 @@ class RestorationPipeline:
         pending = collections.deque()               # (device result kept alive, host view, D2H-done event)
         for i, audio in enumerate(audios):
             k = i % depth
-            if audio.dim() == 1:
-                audio = audio.unsqueeze(0)
-            if audio.dim() != 2 or audio.shape[0] != 1:
-                raise RuntimeError(f"expected mono audio [1, N], got {tuple(audio.shape)}")
+            audio = _as_mono(audio)
             n = audio.shape[1]
-            if n == 0:
-                raise ValueError("empty audio")
             if audio.is_cuda:
                 a = audio
             else:
@@ -348,8 +386,8 @@ class RestorationPipeline:
           chunks than a group holds runs alone.
         * `mode="exact"`: stage 1 (denoise -> super-res) runs the full chunks of all files of a group in shared
           batches; the stereo stage runs the files in lockstep, window j of every file in ONE `forward_window` launch
-          with per-file state positions (`plan_exact_windows`), the LSTM state passed from step to step.  Files
-          shorter than one window run alone.
+          (`plan_exact_windows`), the LSTM state passed from step to step.  Files shorter than one window run alone.
+          `restore(mode="exact")` is this path with one file.
 
         `normalize` applies per file, as in `restore`."""
         for key in ("chunk_range", "reuse_output", "streams"):
@@ -359,38 +397,27 @@ class RestorationPipeline:
             raise TypeError(f"restore_many got unexpected arguments {sorted(excluded)}")
         if mode not in ("chunked", "exact"):
             raise ValueError(f"restore_many: mode must be 'chunked' or 'exact', got {mode!r}")
-        audios = list(audios)
-        if not audios:
+        files = [_as_mono(a) for a in audios]
+        if not files:
             return []
-        was_host = []
-        files = []
         with torch.cuda.device(self.device):
-            for audio in audios:
-                if audio.dim() == 1:
-                    audio = audio.unsqueeze(0)
-                if audio.dim() != 2 or audio.shape[0] != 1:
-                    raise RuntimeError(f"expected mono audio [1, N], got {tuple(audio.shape)}")
-                if audio.shape[1] == 0:
-                    raise ValueError("empty audio")
-                was_host.append(not audio.is_cuda)
-                files.append(audio)
-            run = self._many_chunked if mode == "chunked" else self._many_exact
-            outs = run(files, chunk_size, overlap, batch_chunks, normalize)
-        return [y.cpu() if h and not return_device else y for y, h in zip(outs, was_host)]
+            if mode == "chunked":
+                outs = self._many_chunked(files, chunk_size, overlap, batch_chunks, normalize)
+            else:
+                outs = self._restore_exact([self._prepared(a, normalize) for a in files], chunk_size, batch_chunks)
+                if normalize:
+                    for y in outs:
+                        self._normalize_(y)
+        return [y.cpu() if not a.is_cuda and not return_device else y for y, a in zip(outs, files)]
 
     def _prepared(self, audio, normalize):
-        """Device copy of one mono file, normalised like `restore` normalises it."""
+        """Device copy of one mono `[1,N]` file that the pipeline may overwrite, normalised when `normalize`."""
         a = audio.to(self.device, torch.float32, non_blocking=True).contiguous()
         if a.data_ptr() == audio.data_ptr():
             a = a.clone()
         if normalize:
             self._normalize_(a)
         return a
-
-    def _budget(self):
-        free, _ = torch.cuda.mem_get_info(self.device)
-        held = sum(b.numel() for b in (self._ws or {}).values() if b is not None)
-        return int((free + held) * 0.85)
 
     @staticmethod
     def _packed(sizes, device):
@@ -448,33 +475,35 @@ class RestorationPipeline:
         flush()
         return outs
 
-    def _many_exact(self, files, chunk_size, overlap, batch_chunks, normalize):
-        r, E, P = self.rate, EXACT_STEREO_HALO, EXACT_LSTM_LEAD
+    def _restore_exact(self, ins, chunk_size, batch_chunks):
+        """Whole-file-exact restoration of normalised mono `[1,N]` device signals `ins` -> their `[2, rate*N]`, before
+        output normalisation.  Stage 1 (denoise -> super-res) is `_exact_stage1` with `L = chunk_size` rounded down to a
+        multiple of 8.  The stereo stage cuts each stage-1 signal into the windows of `plan_exact_windows` and runs the
+        files of a group in lockstep (`_exact_group`); a file shorter than one window runs alone, through one stereo
+        forward over its whole stage-1 signal."""
+        r, E = self.rate, EXACT_STEREO_HALO
         Lc = chunk_size - chunk_size % 8
         if Lc < 4 * EXACT_HALO:
             raise ValueError(f"mode='exact' needs chunk_size >= {4 * EXACT_HALO} (conv halos of {EXACT_HALO} samples per chunk edge)")
-        S = (r * Lc - 2 * E) // 16 * 16
+        S = (r * Lc - 2 * E) // 16 * 16                 # kept samples per interior window
         W = S + 2 * E
-        outs = [None] * len(files)
-        plans = [plan_exact_windows(r * a.shape[1], S) for a in files]
+        plans = [plan_exact_windows(r * a.shape[1], S) for a in ins]
+        outs = [None] * len(ins)
         lock = []
         for f, plan in enumerate(plans):
-            if plan is None:                                 # shorter than one window: alone
-                outs[f] = self.restore(files[f], mode="exact", chunk_size=chunk_size, batch_chunks=batch_chunks,
-                                       normalize=normalize, return_device=True)
+            if plan is None:
+                sig = torch.empty((1, 1, r * ins[f].shape[1]), dtype=torch.float32, device=self.device)
+                self._exact_stage1([ins[f]], [sig[0]], Lc, batch_chunks)
+                outs[f] = self.stereo.forward_window(sig)[0][0]
             else:
                 lock.append(f)
         if not lock:
             return outs
-        # groups: up to 16 windows per SM (8, then whatever fits) beside the files' stage-1 signals and outputs
-        sms = torch.cuda.get_device_properties(self.device).multi_processor_count
-        budget = self._budget()
-        per_file = lambda f: 4 * 3 * r * files[f].shape[1]  # stage-1 signal + stereo output
-        cap = 1
-        for per_sm in (16, 8, 2):
-            cap = min(len(lock), per_sm * sms)
-            if self.stereo_workspace_bytes(cap, W) <= budget // 2:
-                break
+        # groups: up to 16 windows per SM (8, then 2) beside the files' stage-1 signals and outputs
+        free, held, sms = self._memory()
+        budget = self._budget(free, held)
+        cap = self._group_cap(len(lock), budget, sms, lambda b: self.stereo_workspace_bytes(b, W))
+        per_file = lambda f: 4 * 3 * r * ins[f].shape[1]    # stage-1 signal + stereo output
         groups, cur, used = [], [], 0
         for f in lock:
             if cur and (len(cur) == cap or used + per_file(f) > budget // 2):
@@ -484,8 +513,8 @@ class RestorationPipeline:
             used += per_file(f)
         groups.append(cur)
         for grp in groups:
-            self._exact_group([files[f] for f in grp], [plans[f] for f in grp], Lc, W, batch_chunks, normalize,
-                              outs, grp)
+            for f, y in zip(grp, self._exact_group([ins[f] for f in grp], [plans[f] for f in grp], Lc, W, batch_chunks)):
+                outs[f] = y
         return outs
 
     def stereo_workspace_bytes(self, batch: int, T: int) -> int:
@@ -494,40 +523,47 @@ class RestorationPipeline:
             _lib.check(_lib.lib().ar_model_workspace_bytes(self.stereo.native_handle(self.device), batch, T, C.byref(need)))
         return need.value
 
-    def _exact_group(self, files, plans, Lc, W, batch_chunks, normalize, outs, idx):
+    def _exact_group(self, ins, plans, Lc, W, batch_chunks):
+        """Stage 1 of the files `ins` in shared batches, then their stereo stage in lockstep: window j of every file
+        (`plans`, from `plan_exact_windows`) in ONE `forward_window` launch, the LSTM state passed from step to step."""
         r, L = self.rate, _lib.lib()
-        Ns = [a.shape[1] for a in files]
-        Ms = [r * n for n in Ns]
+        Ms = [r * a.shape[1] for a in ins]
         sig_all, sig_offs = self._packed(Ms, self.device)
         out_all, out_offs = self._packed([2 * m for m in Ms], self.device)
-        ins = [self._prepared(a, normalize) for a in files]
         self._exact_stage1(ins, [sig_all[o:o + m].view(1, m) for o, m in zip(sig_offs, Ms)], Lc, batch_chunks)
-        # lockstep over windows: files sorted by window count, so the files still running at step j are a prefix and
-        # the state of step j + 1 is the first rows of the state step j returned
-        order = sorted(range(len(files)), key=lambda i: -len(plans[i]))
-        ws = torch.empty(_lib.WINDOW_IO_BYTES_PER_ITEM * len(files), dtype=torch.uint8, device=self.device)
+        # files sorted by window count, so the files still running at step j are a prefix and the state of step j + 1 is
+        # the first rows of the state step j returned
+        order = sorted(range(len(ins)), key=lambda i: -len(plans[i]))
+        ws = torch.empty(_lib.WINDOW_IO_BYTES_PER_ITEM * len(ins), dtype=torch.uint8, device=self.device)
+        n_steps = len(plans[order[0]])
         state = None
-        for j in range(len(plans[order[0]])):
+        for j in range(n_steps):
             act = [i for i in order if len(plans[i]) > j]
             B = len(act)
             wins = [plans[i][j] for i in act]
-            x = torch.empty((B, 1, W), dtype=torch.float32, device=self.device)
+            # window 0 keeps [0, k) and needs EXACT_STEREO_HALO samples right of it: the rest of [0, W) would only be
+            # scanned and discarded, so step 0 runs the windows' first max(k) + EXACT_STEREO_HALO samples
+            T = W if j else max(w[3] for w in wins) + EXACT_STEREO_HALO
+            x = torch.empty((B, 1, T), dtype=torch.float32, device=self.device)
             offs = (C.c_int64 * B)(*[sig_offs[i] + w[0] for i, w in zip(act, wins)])
-            _lib.check(L.ar_gather_windows(sig_all.data_ptr(), sig_all.numel(), offs, B, W, x.data_ptr(), ws.data_ptr(),
+            _lib.check(L.ar_gather_windows(sig_all.data_ptr(), sig_all.numel(), offs, B, T, x.data_ptr(), ws.data_ptr(),
                                            ws.numel(), self._stream()))
+            # no state is handed on after the last step; a position shared by every window that the scalar kernel
+            # accepts (a multiple of 8) goes as an int, per-file positions (window 0's `k - P`) as a list
+            pos = [w[4] for w in wins]
+            if j == n_steps - 1:
+                pos = None
+            elif len(set(pos)) == 1 and pos[0] % 8 == 0:
+                pos = pos[0]
             y, state = self.stereo.forward_window(x, None if state is None else state[:B], lstm_start=wins[0][1],
-                                                  state_pos=[w[4] for w in wins])
+                                                  state_pos=pos)
             dst = []
             for i, w in zip(act, wins):
                 dst += [out_offs[i] + w[0] + w[2], out_offs[i] + Ms[i] + w[0] + w[2]]
-            _lib.check(L.ar_scatter_kept(y.data_ptr(), B, W, (C.c_int64 * (2 * B))(*dst), (C.c_int * B)(*[w[2] for w in wins]),
+            _lib.check(L.ar_scatter_kept(y.data_ptr(), B, T, (C.c_int64 * (2 * B))(*dst), (C.c_int * B)(*[w[2] for w in wins]),
                                          (C.c_int * B)(*[w[3] - w[2] for w in wins]), out_all.data_ptr(), out_all.numel(),
                                          ws.data_ptr(), ws.numel(), self._stream()))
-        for i, (o, m) in enumerate(zip(out_offs, Ms)):
-            y = out_all[o:o + 2 * m].view(2, m)
-            if normalize:
-                self._normalize_(y)
-            outs[idx[i]] = y
+        return [out_all[o:o + 2 * m].view(2, m) for o, m in zip(out_offs, Ms)]
 
     def _exact_stage1(self, ins, sigs, L, batch_chunks):
         """Stage 1 of the whole-file-exact mode (denoise -> super-res) for normalised mono `[1,N]` device signals `ins`
@@ -551,9 +587,8 @@ class RestorationPipeline:
             plans.append((N, n, n if (n - 1) * hop + L <= N else n - 1))
         full = [(f, i) for f, (_, _, n_full) in enumerate(plans) for i in range(n_full)]
         if batch_chunks <= 0:
-            free, _ = torch.cuda.mem_get_info(self.device)
-            sms = torch.cuda.get_device_properties(self.device).multi_processor_count
-            batch_chunks = max(1, min(len(full), 8 * sms, self.max_batch(L, int(free * 0.5))))
+            free, _, sms = self._memory()
+            batch_chunks = self._stage1_batch(len(full), free, sms, self.workspace_bytes(1, L))
         for b0 in range(0, len(full), batch_chunks):
             items = full[b0:b0 + batch_chunks]
             buf = torch.empty((len(items), 1, L), dtype=torch.float32, device=self.device)
@@ -590,47 +625,16 @@ class RestorationPipeline:
                 z = stage1(ins[f][:, start:N].reshape(1, 1, N - start).contiguous())
                 sigs[f][:, r * lo:r * N] = z[0, :, r * (lo - start):r * (N - start)]
 
-    def _restore_exact(self, a, N, chunk_size, batch_chunks):
-        """Whole-file-exact chunked restoration of a normalised mono `[1,N]` device signal -> `[2, rate*N]`.
-
-        Stage 1, denoise (-> super-res): `_exact_stage1` with `L = chunk_size` rounded down to a multiple of 8.
-        Stage 2, stereo: segments of the stage-1 signal with EXACT_STEREO_HALO samples of context on both sides go
-        through `forward_window` one after the other; the scan of segment j starts EXACT_LSTM_LEAD samples before the
-        segment's kept range from the (h, c) its predecessor recorded at exactly that sample."""
-        r, H = self.rate, EXACT_HALO
-        L = chunk_size - chunk_size % 8
-        if L < 4 * H:
-            raise ValueError(f"mode='exact' needs chunk_size >= {4 * H} (conv halos of {H} samples per chunk edge)")
-        sig = torch.empty((1, r * N), dtype=torch.float32, device=self.device)
-        self._exact_stage1([a], [sig], L, batch_chunks)
-
-        M, E, P = r * N, EXACT_STEREO_HALO, EXACT_LSTM_LEAD
-        S2 = (r * L - 2 * E) // 16 * 16                 # kept samples per stereo segment
-        out = torch.empty((2, M), dtype=torch.float32, device=self.device)
-        state = None
-        n_seg = -(-M // S2)
-        for j in range(n_seg):
-            a0, a1 = j * S2, min(M, (j + 1) * S2)
-            e0, e1 = max(0, a0 - E), min(M, a1 + E)
-            last = j == n_seg - 1
-            y, state = self.stereo.forward_window(sig[:, e0:e1].reshape(1, 1, e1 - e0).contiguous(), state,
-                                                  lstm_start=0 if j == 0 else a0 - P - e0,
-                                                  state_pos=None if last else a1 - P - e0)
-            out[:, a0:a1] = y[0, :, a0 - e0:a1 - e0]
-        return out
-
     def check_dynamic_range(self, audio: torch.Tensor, chunk_size: int = DEFAULT_CHUNK, max_chunks: int = 8) -> dict:
         """Dynamic-range audit of this checkpoint set on `audio` (`[1,N]`, any device; normalised here like `restore`
         does): runs the three models layer by layer on up to `max_chunks` chunks -- evenly spread over the file plus the
         one holding the global peak -- and returns `{"<model>.<layer>": max |activation|}`.  Inter-layer activations
         are stored in fp16 and saturate at +-65504; raises RuntimeError naming the layer if one clipped
         (INTEGRATION.md, "dynamic range")."""
-        if audio.dim() == 1:
-            audio = audio.unsqueeze(0)
+        audio = _as_mono(audio)
         N = audio.shape[1]
         with torch.cuda.device(self.device), torch.no_grad():
-            a = audio.to(self.device, torch.float32).contiguous().clone()
-            self._normalize_(a)
+            a = self._prepared(audio, True)
             T = min(chunk_size, N)
             n = max(1, N // T)
             picks = sorted(set([int(k * (n - 1) / max(1, max_chunks - 2)) for k in range(max_chunks - 1)] if n > 1 else [0])
@@ -667,34 +671,29 @@ class RestorationPipeline:
         y_all = torch.empty((cnt_all, 2, r * chunk_size), dtype=torch.float32, device=self.device)
         firsts = list(range(c0, hi, batch_chunks))
         n_streams = max(1, min(streams, len(firsts)))
+        # Batches of chunks are independent: with several streams they are issued round-robin on side streams (own
+        # workspace each), so the latency-bound LSTM scan of one batch runs under the tensor-core convs of the next.
         main = torch.cuda.current_stream(self.device)
-        if n_streams == 1:
-            buf = torch.empty((min(batch_chunks, cnt_all), 1, chunk_size), dtype=torch.float32, device=self.device)
-            for first in firsts:
-                cnt = min(batch_chunks, hi - first)
-                _lib.check(L.ar_split_chunks(a.data_ptr(), N, buf.data_ptr(), first, cnt, chunk_size, overlap, self._stream()))
-                self.forward_chunks(buf[:cnt], y_all[first - c0:first - c0 + cnt])
-        else:
-            # Batches of chunks are independent: issue them round-robin on side streams (own workspace each)
-            # so the latency-bound LSTM scan of one batch runs under the tensor-core convs of the next.
-            side = self._side_streams(n_streams)
+        run_on = self._side_streams(n_streams) if n_streams > 1 else [main]
+        if n_streams > 1:
             ready = torch.cuda.Event()
             ready.record(main)
-            bufs = [torch.empty((min(batch_chunks, cnt_all), 1, chunk_size), dtype=torch.float32, device=self.device)
-                    for _ in range(n_streams)]
-            for j, first in enumerate(firsts):
-                k = j % n_streams
-                cnt = min(batch_chunks, hi - first)
-                if j < n_streams:
-                    side[k].wait_event(ready)
-                with torch.cuda.stream(side[k]):
-                    _lib.check(L.ar_split_chunks(a.data_ptr(), N, bufs[k].data_ptr(), first, cnt, chunk_size, overlap,
-                                                 side[k].cuda_stream))
-                    self.forward_chunks(bufs[k][:cnt], y_all[first - c0:first - c0 + cnt], slot=k)
-            for st in side:
+            for st in run_on:
+                st.wait_event(ready)
+        bufs = [torch.empty((min(batch_chunks, cnt_all), 1, chunk_size), dtype=torch.float32, device=self.device)
+                for _ in range(n_streams)]
+        for j, first in enumerate(firsts):
+            k = j % n_streams
+            cnt = min(batch_chunks, hi - first)
+            with torch.cuda.stream(run_on[k]):
+                _lib.check(L.ar_split_chunks(a.data_ptr(), N, bufs[k].data_ptr(), first, cnt, chunk_size, overlap,
+                                             self._stream()))
+                self.forward_chunks(bufs[k][:cnt], y_all[first - c0:first - c0 + cnt], slot=k)
+        if n_streams > 1:
+            for st in run_on:
                 main.wait_stream(st)
             for t in bufs + [a, y_all]:
-                for st in side:
+                for st in run_on:
                     t.record_stream(st)
         # stitch chunks [c0, hi) as a virtual file, then keep this shard's span [lo*hop, hi*hop) (or to N)
         n_virtual = N - c0 * hop if hi == n_chunks else (cnt_all - 1) * hop + chunk_size
@@ -720,21 +719,13 @@ def restore_sharded(pipes, audio: torch.Tensor, chunk_size: int = DEFAULT_CHUNK,
     on the host) equals `pipes[0].restore(audio, mode="chunked", ...)`."""
     if not pipes:
         raise ValueError("restore_sharded: no pipelines")
-    if audio.dim() == 1:
-        audio = audio.unsqueeze(0)
-    if audio.dim() != 2 or audio.shape[0] != 1:
-        raise RuntimeError(f"expected mono audio [1, N], got {tuple(audio.shape)}")
-    N = audio.shape[1]
-    n_chunks = len(plan_chunks(N, chunk_size, overlap))
+    audio = _as_mono(audio)
+    n_chunks = len(plan_chunks(audio.shape[1], chunk_size, overlap))
     world = min(len(pipes), n_chunks)
     head = pipes[0]
     was_host = not audio.is_cuda
     with torch.cuda.device(head.device):
-        a = audio.to(head.device, torch.float32).contiguous()
-        if a.data_ptr() == audio.data_ptr():
-            a = a.clone()
-        if normalize:
-            head._normalize_(a)
+        a = head._prepared(audio, normalize)
         torch.cuda.current_stream(head.device).synchronize()     # the peers read `a` on their own streams
     parts = []
     for r in range(world):
@@ -856,15 +847,7 @@ def restore_audio(
     else:
         audio, _ = load_audio(input_path, sample_rate=sample_rate, mono=True)
         audio = audio.pin_memory()
-    print("Loading denoiser model...")
-    den = _load_checkpoint(AudioDenoiser(), denoiser_checkpoint, device)
-    sr = None
-    if enable_super_resolution:
-        print("Loading super-resolution model...")
-        sr = _load_checkpoint(AudioSuperResolution(upscale_factor=2), super_res_checkpoint, device)
-    print("Loading stereo separator model...")
-    st = _load_checkpoint(StereoSeparator(), stereo_checkpoint, device)
-    pipe = RestorationPipeline(den, sr, st, device)
+    pipe = _load_pipeline(denoiser_checkpoint, super_res_checkpoint, stereo_checkpoint, enable_super_resolution, device)
     pipe.check_dynamic_range(audio, chunk_size)      # raises if this checkpoint clips the fp16 activation storage
     print("Applying denoising...")
     if enable_super_resolution:
@@ -891,15 +874,7 @@ def _restore_directory(input_dir, output_dir, denoiser_checkpoint, super_res_che
     print(f"Processing directory: {input_dir} ({len(names)} files)")
     print(f"Device: {device}")
     os.makedirs(output_dir, exist_ok=True)
-    print("Loading denoiser model...")
-    den = _load_checkpoint(AudioDenoiser(), denoiser_checkpoint, device)
-    sr = None
-    if enable_super_resolution:
-        print("Loading super-resolution model...")
-        sr = _load_checkpoint(AudioSuperResolution(upscale_factor=2), super_res_checkpoint, device)
-    print("Loading stereo separator model...")
-    st = _load_checkpoint(StereoSeparator(), stereo_checkpoint, device)
-    pipe = RestorationPipeline(den, sr, st, device)
+    pipe = _load_pipeline(denoiser_checkpoint, super_res_checkpoint, stereo_checkpoint, enable_super_resolution, device)
     t0 = time.perf_counter()
     audios, t_audit = [], 0.0
     for n in names:

@@ -146,6 +146,26 @@ def test_shard_range_partitions():
             assert max(sizes) - min(sizes) <= 1
 
 
+def test_exact_mode_memory_rules():
+    """The memory rules of mode="exact" on fake device states (free bytes, cached workspace bytes, SMs): the stage-1 batch
+    (up to 8 chunks per SM within half the free memory) and the lockstep group cap (16, 8 or 2 windows per SM, the first
+    whose stereo workspace fits in half of 85 % of free + cached)."""
+    from ml_audio_restoration_b200 import RestorationPipeline as P
+    GB = 1 << 30
+    stereo_ws = lambda b: 4096 + 30_000_000 * b          # bytes of a stereo window launch of b windows
+    cases = [  # free, held, sms, n_files -> budget, group cap; n_chunks, chunk_ws -> stage-1 batch
+        (170 * GB, 0, 148, 5000, 155_155_693_568, 2368, 9000, 50_000_000, 1184),    # 16 windows per SM fit
+        (90 * GB, 10 * GB, 148, 5000, 91_268_055_040, 1184, 9000, 150_000_000, 322),  # 8 per SM; memory bounds stage 1
+        (20 * GB, 3 * GB, 148, 5000, 20_991_652_659, 296, 9000, 50_000_000, 214),     # 2 per SM
+        (170 * GB, 0, 148, 3, 155_155_693_568, 3, 5, 50_000_000, 5),                # fewer files / chunks than a launch
+        (1 * GB, 0, 8, 100, 912_680_550, 16, 40, 10 * GB, 1),                       # nothing fits: 2 per SM, 1 chunk
+    ]
+    for free, held, sms, n_files, budget, cap, n_chunks, chunk_ws, batch in cases:
+        assert P._budget(free, held) == budget
+        assert P._group_cap(n_files, budget, sms, stereo_ws) == cap
+        assert P._stage1_batch(n_chunks, free, sms, chunk_ws) == batch
+
+
 def test_wav_round_trip(tmp_path):
     from ml_audio_restoration_b200 import load_audio, save_audio
     a = 0.5 * torch.sin(torch.arange(4410.0) * 0.05)[None].repeat(2, 1)
